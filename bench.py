@@ -8,7 +8,7 @@ one synthetic batch:
     QP build (discretise A,B per speed, delta-u augmentation, layout) -> Ruiz scaling + cached KKT factorisation
     -> ADMM to convergence -> gather of the control sequences (+ NCCL all_gather of them at N > 1).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--records all|none|a,b,..]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--records all|none|a,b,..] [--dump-outputs DIR]
 
 value   : whole-job QP solves/sec with the inputs already resident in HBM (weak scaling: 65536 QPs per GPU)
 e2e     : the same through the public API (LateralMPC.solve_batch) from pinned HOST buffers, H2D of the inputs, the
@@ -45,7 +45,8 @@ ALL_RECORDS = ("strong", "qp_build", "configs1", "configs3", "configs4", "fp32")
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5,
+                    help="timed steps of the headline and of its e2e figure (the records keep their own step counts)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--batch", type=int, default=65536, help="QPs per GPU (weak scaling)")
@@ -58,11 +59,38 @@ def parse():
     ap.add_argument("--records", default="all", help="all | none | comma-separated subset of " + ",".join(ALL_RECORDS))
     ap.add_argument("--sweep-scenarios", type=int, default=131072, help="configs4: closed-loop scenarios per GPU")
     ap.add_argument("--sweep-steps", type=int, default=200, help="configs4: closed-loop steps")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the headline returned to its caller as DIR/<name>.npy: u (the control "
+                         "sequences; at N > 1 every rank's, rank by rank), iter, status_val, pri_res, dua_res (rank 0's QPs); "
+                         "float32 or float64, at most 64 MB in all (beyond that one fixed, seeded sample of QPs in every array)")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return a
 
 
 def host_cores():
     return len(os.sched_getaffinity(0))
+
+
+DUMP_BYTES = 63 * 10 ** 6          # --dump-outputs: at most 64 MB in all, .npy headers included
+
+
+def dump_outputs(d, arrays, seed=0):
+    """np.save of each array as d/<name>.npy, float32 kept, anything else as float64.  Every array holds n rows (one per QP)
+    or k blocks of n rows (at N > 1, u: one block per rank, in rank order).  Arrays that together exceed DUMP_BYTES keep the
+    same QPs: one sorted sample r of the n rows, drawn with a fixed seed (the same from run to run), from every block."""
+    os.makedirs(d, exist_ok=True)
+    arrays = {k: np.asarray(v, dtype=np.float32 if v.dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_BYTES:
+        n = min(v.shape[0] for v in arrays.values())
+        r = np.sort(np.random.default_rng(seed).choice(n, max(1, n * DUMP_BYTES // total), replace=False))
+        arrays = {k: v.reshape(-1, n, *v.shape[1:])[:, r].reshape(-1, *v.shape[1:]) for k, v in arrays.items()}
+    for k, v in arrays.items():
+        np.save(os.path.join(d, k + ".npy"), v)
 
 
 def workload_config(a, n_gpus):
@@ -345,7 +373,7 @@ def run_ours(a):
     wall0 = time.perf_counter()
     ev[0].record()
     for i in range(a.steps):
-        res, _ = step(a.warmup + i)
+        res, u_all = step(a.warmup + i)
         it_buf[i].copy_(res.info.iter); st_buf[i].copy_(res.info.status_val)
         ev[i + 1].record()
     drain()
@@ -353,6 +381,11 @@ def run_ours(a):
     end_ev.record()
     barrier()
     wall1 = time.perf_counter()
+    if a.dump_outputs and rank == 0:
+        # the last step's results are views of the solver's reused buffers: copied out before any later solve
+        inf = res.info
+        dump_outputs(a.dump_outputs, {"u": u_all.cpu().numpy(), "iter": inf.iter.cpu().numpy(), "status_val": inf.status_val.cpu().numpy(),
+                                      "pri_res": inf.pri_res.cpu().numpy(), "dua_res": inf.dua_res.cpu().numpy()})
     launches = be.launch_count() - launches0
     step_ms = [ev[i].elapsed_time(ev[i + 1]) for i in range(a.steps)]
     total_ms = ev[0].elapsed_time(end_ev)

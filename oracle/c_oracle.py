@@ -1,14 +1,10 @@
 """ORACLE — test infrastructure only.  ctypes front-end of oracle/osqp_admm.c."""
 import ctypes as C
-import hashlib
-import os
-import subprocess
 
 import numpy as np
 import scipy.sparse as sp
 
-_HERE = os.path.dirname(os.path.abspath(__file__))
-_SO = os.path.join(_HERE, "_build", "liboracle_osqp.so")
+from .library import build
 
 
 class Settings(C.Structure):
@@ -20,29 +16,6 @@ class Settings(C.Structure):
 
 class Info(C.Structure):
     _fields_ = [("iter", C.c_int), ("status", C.c_int), ("pri_res", C.c_double), ("dua_res", C.c_double)]
-
-
-def _stamp():
-    """Content hash of the source, the build recipe and the host CPU (the library is built with -march=native and
-    travels with the repo snapshot: a different host must rebuild it)."""
-    h = hashlib.sha256()
-    for f in ("osqp_admm.c", "Makefile"):
-        h.update(open(os.path.join(_HERE, f), "rb").read())
-    try:
-        cpu = [l for l in open("/proc/cpuinfo") if l.startswith(("model name", "flags"))][:2]
-    except OSError:
-        cpu = []
-    h.update("".join(cpu).encode())
-    return h.hexdigest()
-
-
-def build(force=False):
-    stamp = os.path.join(_HERE, "_build", "liboracle_osqp.sha256")
-    want = _stamp()
-    if force or not os.path.exists(_SO) or not os.path.exists(stamp) or open(stamp).read() != want:
-        subprocess.check_call(["make", "-s", "-B", "-C", _HERE])
-        open(stamp, "w").write(want)
-    return _SO
 
 
 _lib = None

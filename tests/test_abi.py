@@ -32,7 +32,9 @@ def test_header_binding_and_library_agree():
 
 def test_library_is_compiled_for_sm_100a():
     import subprocess
-    out = subprocess.run(["cuobjdump", "-lelf", g.build_cuda()], capture_output=True, text=True).stdout
+    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")        # the toolkit build_cuda() compiles with
+    out = subprocess.run([os.path.join(os.path.dirname(nvcc), "cuobjdump"), "-lelf", g.build_cuda()], capture_output=True,
+                         text=True).stdout
     assert "sm_100a" in out
 
 

@@ -248,6 +248,31 @@ def test_full_size_batch_properties(cuda_backend):
     assert float((dmax - du)[ybu > ytol].max()) < 2e-3 and float((du + dmax)[ybu < -ytol].max()) < 2e-3
 
 
+def test_bench_dump_outputs_are_the_last_timed_step(cuda_backend, tmp_path):
+    """`bench.py --dump-outputs`, twice with the same arguments: identical files, holding what LateralMPC.solve_batch returns
+    for the inputs of the last timed step (--warmup 1 --steps 1: the headline's batch of seed 1)."""
+    import os, subprocess, sys
+    from python_mpc_b200 import workloads
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    names = ("u", "iter", "status_val", "pri_res", "dua_res")
+    out = []
+    for d in ("a", "b"):
+        p = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--batch", "256", "--steps", "1", "--warmup", "1",
+                            "--records", "none", "--no-cpu-baseline", "--dump-outputs", str(tmp_path / d)],
+                           capture_output=True, text=True, timeout=600, cwd=root)
+        assert p.returncode == 0, p.stderr[-2000:]
+        assert sorted(os.listdir(tmp_path / d)) == sorted(n + ".npy" for n in names)
+        out.append({n: np.load(tmp_path / d / (n + ".npy")) for n in names})
+    for n in names:
+        assert out[0][n].dtype == np.float64 and np.array_equal(out[0][n], out[1][n]), n
+    wl = workloads.lateral_slack_increment(256, seed=1, dtype=torch.float64)
+    r = wl.make_controller(rho=5.0, eps_abs=1e-4, eps_rel=1e-4, warm_start=False).solve_batch(wl.x0, wl.xr, wl.speed, want_x=False)
+    u = r.u.cpu().numpy()
+    assert out[0]["u"].shape == u.shape == (256, 20, 1)
+    assert np.array_equal(out[0]["iter"], r.info.iter.cpu().numpy()) and (out[0]["status_val"] == 1).all()
+    assert np.abs(out[0]["u"] - u).max() <= 1e-10 * np.abs(u).max()
+
+
 def test_rate_bounds_hold_at_full_size(cuda_backend):
     from python_mpc_b200 import workloads
     wl = workloads.lateral_slack_increment(65536, seed=5, dtype=torch.float64)

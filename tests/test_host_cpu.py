@@ -115,3 +115,24 @@ def test_bench_reference_arm_emits_the_contract_line():
     out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--impl", "reference", "--gpus", "2", "--batch", "512",
                           "--steps", "1", "--warmup", "0"], capture_output=True, text=True, timeout=120, cwd=root, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+def test_bench_dump_outputs_are_float_bounded_and_repeatable(tmp_path, monkeypatch):
+    """`bench.py --dump-outputs`: float32 / float64 .npy files; beyond the size bound one sample of QPs, the same in every array
+    (u of two ranks: the same QPs of each rank's block) and in every run."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 100000)
+    arrays = {"u": np.arange(2000 * 20, dtype=np.float64).reshape(2000, 20, 1), "iter": np.arange(1000, dtype=np.int32),
+              "pri_res": np.arange(1000, dtype=np.float32)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    out = {k: np.load(tmp_path / "a" / (k + ".npy")) for k in arrays}
+    assert out["u"].dtype == np.float64 and out["iter"].dtype == np.float64 and out["pri_res"].dtype == np.float32
+    assert sum(v.nbytes for v in out.values()) <= 100000 and 0 < out["iter"].size < 1000
+    qps = out["iter"].astype(int)
+    assert (np.diff(qps) > 0).all() and np.array_equal(out["pri_res"], qps)
+    assert np.array_equal(out["u"], arrays["u"][np.concatenate([qps, 1000 + qps])])   # rank 0's QPs, then the same of rank 1
+    for k in arrays:
+        assert np.array_equal(out[k], np.load(tmp_path / "b" / (k + ".npy")))
+    bench.dump_outputs(str(tmp_path / "c"), {"iter": arrays["iter"]})             # within the bound: everything
+    assert np.array_equal(np.load(tmp_path / "c" / "iter.npy"), arrays["iter"])

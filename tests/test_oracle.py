@@ -33,6 +33,39 @@ def test_osqp_documented_demo_qp():
     np.testing.assert_allclose(x, r.x, atol=1e-12)
 
 
+@pytest.mark.parametrize("shared_dir", ["absent", "world_writable", "foreign_owner"])
+def test_stale_oracle_in_a_read_only_tree_is_rebuilt_outside_it(tmp_path, monkeypatch, shared_dir):
+    """bench.py may run from a tree it cannot write: a missing or stale library is then built in a per-user temporary
+    directory, reused while current — and never loaded from that directory when another user could have written it."""
+    import ctypes
+    import os
+    import tempfile
+    from oracle import library
+    monkeypatch.setattr(library, "SO", str(tmp_path / "tree" / "liboracle_osqp.so"))
+    monkeypatch.setattr(library, "_writable", lambda d: False)
+    (tmp_path / "tmp").mkdir()
+    monkeypatch.setattr(tempfile, "tempdir", str(tmp_path / "tmp"))
+    uid = os.getuid()
+    if shared_dir == "foreign_owner":
+        monkeypatch.setattr(os, "getuid", lambda: uid + 1)              # the directory below belongs to "another" user
+    planted = tmp_path / "tmp" / ("mpcb_oracle_%d_%s" % (os.getuid(), library._stamp()[:16]))
+    if shared_dir != "absent":
+        planted.mkdir(mode=0o700)
+        (planted / "liboracle_osqp.so").write_bytes(b"planted")
+        (planted / "liboracle_osqp.sha256").write_text(library._stamp())
+        if shared_dir == "world_writable":
+            planted.chmod(0o777)
+    so = library.build()
+    assert so.startswith(str(tmp_path / "tmp")) and not (tmp_path / "tree").exists()
+    assert hasattr(ctypes.CDLL(so), "oracle_osqp_solve")
+    if shared_dir == "absent":
+        assert os.path.dirname(so) == str(planted) and planted.stat().st_mode & 0o777 == 0o700
+        mtime = os.path.getmtime(so)
+        assert library.build() == so and os.path.getmtime(so) == mtime      # up to date: found again, not rebuilt
+    else:
+        assert os.path.dirname(so) != str(planted) and (planted / "liboracle_osqp.so").read_bytes() == b"planted"
+
+
 def test_restated_assembly_equals_reference_slack_increment(golden):
     g = golden["lateral_slack_increment_closed_loop"]
     p = ref_qp.qp_slack_increment(g["Ad"], g["Bd"], np.array([0., 0., 5 * DEG, 3., 0.]), np.zeros(4),
