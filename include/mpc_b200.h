@@ -183,14 +183,10 @@ int mpcb_to_element_major(int dtype, int batch, int elems, size_t ld, const void
 int mpcb_to_batch_major(int dtype, int batch, int elems, size_t ld, const void* src, void* dst_rowmajor, void* stream);
 
 /* Process-wide tunables (also read once from the environment: MPCB_NO_TMA, MPCB_NO_RETILE, MPCB_RETILE_MIN_BATCH,
- * MPCB_NO_CERT, MPCB_NO_WIDE, MPCB_NO_DENSE, MPCB_NO_CTA, MPCB_NO_WARP_SETUP):
+ * MPCB_NO_CERT, MPCB_NO_DENSE, MPCB_NO_CTA, MPCB_NO_WARP_SETUP):
  *   "tma"              1 (default) warp-per-tile ADMM kernel with TMA-staged stage records; 0: one lane per QP from global memory
  *   "retile"           1 (default) run the ADMM loop in chunks and re-tile unconverged QPs; 0: one asynchronous launch
  *   "retile_min_batch" smallest batch that is run in chunks (default 4096)
- *   "wide"             1 (default) run the steady-state iterations of small sets (the stragglers after a re-tiling, batches
- *                      below retile_min_batch; at most 4608 QPs — 16384 with per-stage models —, shapes with nx + nu <= 8) with 8 lanes
- *                      per QP
- *                      (admm_wide.cuh); 0: everything in the main kernel.  The two agree to the last bits (not bitwise).
  *   "dense"            1 (default) a batch that shares ONE KKT matrix (shared_model, identical Ruiz scaling of every QP, f64,
  *                      (N+1)(nx+nu) <= 128) runs its steady-state iterations as a dense FP64 tensor-core GEMM with the
  *                      explicit inverse of the reduced KKT matrix (admm_dense.cuh); 0: the per-QP kernels

@@ -10,8 +10,7 @@
 //                     together and meet at a CTA barrier once per iteration (instruction-cache sharing).
 //   Both drive the same stage functions (qp_thread.cuh): forward / backward sweep (first-iteration and save-old
 //   variants as template instantiations) and ONE termination-sweep body that serves the residuals and, on a second
-//   pass over (dx, dy), the infeasibility certificates.  admm_wide.cuh holds the 8-lanes-per-QP variant of the sweeps
-//   for small sets.
+//   pass over (dx, dy), the infeasibility certificates.
 #pragma once
 #include "qp_thread.cuh"
 #include <type_traits>

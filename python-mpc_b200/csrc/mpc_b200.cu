@@ -19,7 +19,6 @@ std::atomic<long long> g_launches{0};
 std::atomic<int> g_opt_tma{std::getenv("MPCB_NO_TMA") ? 0 : 1};
 std::atomic<int> g_opt_retile{std::getenv("MPCB_NO_RETILE") ? 0 : 1};
 std::atomic<int> g_opt_cert{std::getenv("MPCB_NO_CERT") ? 0 : 1};
-std::atomic<int> g_opt_wide{std::getenv("MPCB_NO_WIDE") ? 0 : 1};
 std::atomic<int> g_opt_dense{std::getenv("MPCB_NO_DENSE") ? 0 : 1};
 std::atomic<int> g_opt_cta{std::getenv("MPCB_NO_CTA") ? 0 : 1};
 std::atomic<int> g_opt_warp_setup{std::getenv("MPCB_NO_WARP_SETUP") ? 0 : 1};
@@ -79,7 +78,6 @@ int mpcb_set_option(const char* name, int value) {
     if (n == "tma") g_opt_tma = value != 0;
     else if (n == "retile") g_opt_retile = value != 0;
     else if (n == "certificates") g_opt_cert = value != 0;
-    else if (n == "wide") g_opt_wide = value != 0;
     else if (n == "dense") g_opt_dense = value != 0;
     else if (n == "warp_setup") g_opt_warp_setup = value != 0;
     else if (n == "cta") g_opt_cta = value < 0 ? 0 : (value > 2 ? 2 : value);

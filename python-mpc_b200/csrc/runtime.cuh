@@ -22,7 +22,7 @@ using namespace mpcb;
 // compiled (shape, dtype) plus the ABI layer — see __graft_entry__.build_cuda)
 namespace mpcb_rt {
 extern std::atomic<long long> g_launches;
-extern std::atomic<int> g_opt_tma, g_opt_retile, g_opt_cert, g_opt_wide, g_opt_dense, g_opt_cta, g_opt_warp_setup, g_opt_retile_min;
+extern std::atomic<int> g_opt_tma, g_opt_retile, g_opt_cert, g_opt_dense, g_opt_cta, g_opt_warp_setup, g_opt_retile_min;
 int fail(int code, const std::string& msg);      // records the message for mpcb_last_error(), returns `code`
 }
 struct ShapeOps;

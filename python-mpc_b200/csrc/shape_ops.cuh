@@ -7,7 +7,6 @@
 #include <chrono>
 #include "runtime.cuh"
 #include "admm_kernel.cuh"
-#include "admm_wide.cuh"
 #include "admm_dense.cuh"
 #include "admm_cta.cuh"
 #include "setup_warp.cuh"
@@ -197,33 +196,6 @@ static int launch_admm(const KParams<T>& p, mpcb_solver* s, rt_stream st) {
     return launch_qp<AdmmOp, T, L>(p, st);
 }
 
-#ifdef MPCB_EMU
-constexpr int WIDE_G_HOST = 0;       // tests/emu has no warp shuffles: the wide kernel does not exist there
-#else
-constexpr int WIDE_G_HOST = WIDE_G;
-#endif
-// Steady-state iterations it0+1 .. it_stop of a small, re-tiled set with 8 lanes per QP (admm_wide.cuh).  Returns 1 when
-// the shape / problem flavour is not covered (the caller then lets admm_tma_kernel run those iterations), -1 on error.
-template <typename T, typename L>
-static int launch_wide(const KParams<T>& p, rt_stream st) {
-#ifndef MPCB_EMU
-    if constexpr (L::NW <= WIDE_G) {
-        // worth it while the set is small: ~2400 QPs fill the GPU at 53 us per iteration (45 QP-iterations/us beyond that);
-        // the main kernel needs 104 us per iteration up to ~28000 QPs — the two cross near 4700 QPs
-        // (per-stage models are not staged by the main kernel — its model loads are exposed latency — so there the wide
-        // kernel wins up to much larger sets)
-        if (g_opt_wide.load() == 0 || p.it0 < 1 || p.B > (p.tv ? 16384 : 4608)) return 1;
-        const int threads = 128, per_cta = threads / WIDE_G;
-        if (p.tv) admm_wide_kernel<T, L, true><<<(p.B + per_cta - 1) / per_cta, threads, 0, st>>>(p);
-        else admm_wide_kernel<T, L, false><<<(p.B + per_cta - 1) / per_cta, threads, 0, st>>>(p);
-        ++g_launches;
-        return rt_launch_check("admm_wide") ? -1 : 0;
-    }
-#endif
-    (void)p; (void)st;
-    return 1;
-}
-
 // ---- CTA-per-tile kernel (admm_cta.cuh) ------------------------------------------------------------------------------
 #ifndef MPCB_EMU
 template <typename T, typename L>
@@ -288,9 +260,9 @@ static bool cta_applicable(const mpcb_solver* s, const KParams<T>& p) {
 }
 // Which solves go to admm_cta_kernel: time-varying problems; time-invariant batches that fit the GPU in one wave of CTAs
 // (two per SM: 9472 QPs on 148 SMs) — below that the warp-per-tile kernel runs at one or two warps per SM, 104 us per
-// iteration, and the 8-lanes kernel at 53 us; the CTA kernel needs 45 us per iteration up to one tile per SM and ~65 us at
-// two (scripts/strong_probe.py: 4.7 vs 5.3 ms per step at 256..2048 QPs, 4.7 vs 8.1 ms at 4096, 7.0 vs 8.7 ms at 8192; a
-// second wave loses: 11.6 vs ~9 ms at 10240); everything with "cta" = 2.
+// iteration; the CTA kernel needs 45 us per iteration up to one tile per SM and ~65 us at two (scripts/strong_probe.py:
+// 4.7 vs 5.3 ms per step at 256..2048 QPs, 4.7 vs 8.1 ms at 4096, 7.0 vs 8.7 ms at 8192; a second wave loses: 11.6 vs
+// ~9 ms at 10240); everything with "cta" = 2.
 template <typename T, typename L>
 static bool cta_planned(const mpcb_solver* s, int B, bool tv, int check_every) {
     const int opt = g_opt_cta.load();
@@ -526,13 +498,37 @@ static int ensure_scratch(mpcb_solver* s, int n_unc, size_t mdl_per_qp_bytes) {
     }
     return 0;
 }
+// The set of QPs a chunked host loop iterates on: the whole batch in the home workspace until the first compaction, then
+// the survivors in dense tiles of the scratch workspace (map[j] = home slot of scratch slot j).
+template <typename T, typename L>
+struct LoopSet {
+    int n;                        // QPs in the set
+    int which = 0;                // the next launch lists the set's survivors in s->surv[which]
+    const int* map = nullptr;     // null while the set is the home workspace
+    // Compact the n_unc survivors listed by the last launch into the scratch workspace — records, headers and, when
+    // mdl_per (bytes per QP) is not 0, the staged stage models — and point p at them.  Compaction always reads the home
+    // workspace: a set that already sits in the scratch workspace is copied home first.
+    int compact(mpcb_solver* s, KParams<T>& p, int n_unc, size_t mdl_per, rt_stream st) {
+        if (int r = copy_home(s, st)) return r;
+        if (int r = ensure_scratch(s, n_unc, mdl_per)) return r;
+        if (int r = retile_impl<T>(s, n_unc, s->surv[which], st)) return r;
+        if (mdl_per) if (int r = retile_model<T, L>(s, n_unc, s->surv[which], st)) return r;
+        map = s->surv[which];
+        which ^= 1;               // the next launches list their survivors in the other buffer
+        n = n_unc;
+        p.rec = (T*)s->rec2; p.hdr = (T*)s->hdr2; p.yrows = (T*)s->yrows2;
+        if (mdl_per) p.mdl = (const T*)s->mdl2;
+        return 0;
+    }
+    // x, z, y of a compacted set back to their home columns
+    int copy_home(mpcb_solver* s, rt_stream st) const { return map ? untile_impl<T>(s, n, map, st) : 0; }
+};
 
 // The host loop of the CTA-per-tile kernel.  Small sets: ONE launch, termination tests included, nothing to read back.
 // Large sets: one launch per check interval; after each the number of unsolved QPs is read back, and every time at
 // most four fifths of the current set are left the survivors are compacted into dense tiles of the scratch workspace (their
 // records, headers and staged stage models) — a tile streams 32 QPs' records until its slowest QP terminates, and the
-// iteration counts of a batch spread widely (configs[3]: 150 .. 450).  Compaction always reads the home workspace:
-// a set that already sits in the scratch workspace is copied home first.
+// iteration counts of a batch spread widely (configs[3]: 150 .. 450).
 template <typename T, typename L>
 static int run_cta_loop(mpcb_solver* s, KParams<T> p, int max_iter, int check_every, bool chunked, rt_stream st) {
 #ifndef MPCB_EMU
@@ -542,13 +538,12 @@ static int run_cta_loop(mpcb_solver* s, KParams<T> p, int max_iter, int check_ev
     }
     const int retile_floor = 1024;          // (fewer QPs than this leave most SMs idle either way: compaction buys nothing)
     const size_t mdl_per = p.tv ? (size_t)(p.N + 1) * CtaModel<L>::COUNT * sizeof(T) : 0;
-    int it0 = 0, n_cur = p.B, which = 0;
-    bool in_scratch = false;
-    const int* scratch_map = nullptr;
+    int it0 = 0;
+    LoopSet<T, L> set{p.B};
     const bool trace = std::getenv("MPCB_TRACE") != nullptr;
     const auto t_start = std::chrono::steady_clock::now();
     while (it0 < max_iter) {
-        p.B = n_cur; p.survivors = s->surv[which]; p.qp_map = in_scratch ? scratch_map : nullptr;
+        p.B = set.n; p.survivors = s->surv[set.which]; p.qp_map = set.map;
         p.it0 = it0; p.it_stop = it0 + check_every < max_iter ? it0 + check_every : max_iter; p.list_survivors = 1;
         const int rc = launch_cta<T, L>(p, s, st);
         if (rc != 0) return rc;
@@ -557,23 +552,13 @@ static int run_cta_loop(mpcb_solver* s, KParams<T> p, int max_iter, int check_ev
         if (int r = rt_d2h(&n_unc, s->n_surv, sizeof(int), st)) return -1;
         if (int r = rt_sync(st)) return -1;
         if (int r = rt_memset(s->n_surv, 0, sizeof(int), st)) return -1;
-        if (trace) std::fprintf(stderr, "[mpcb] cta ..%d n=%d -> %d unsolved (scratch=%d)  t=%.3f ms\n", it0, n_cur, n_unc, (int)in_scratch,
+        if (trace) std::fprintf(stderr, "[mpcb] cta ..%d n=%d -> %d unsolved (scratch=%d)  t=%.3f ms\n", it0, set.n, n_unc, (int)(set.map != nullptr),
                                 std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - t_start).count());
         if (n_unc == 0 || it0 >= max_iter) break;
-        if (5 * n_unc <= 4 * n_cur && n_cur >= retile_floor) {      // a fifth of the tiles to gain: worth the two copies
-            if (in_scratch) if (untile_impl<T>(s, n_cur, scratch_map, st)) return -1;
-            if (ensure_scratch(s, n_unc, mdl_per)) return -1;
-            if (retile_impl<T>(s, n_unc, s->surv[which], st)) return -1;
-            if (p.tv) if (retile_model<T, L>(s, n_unc, s->surv[which], st)) return -1;
-            scratch_map = s->surv[which];
-            which ^= 1;                       // the next launches list their survivors in the other buffer
-            in_scratch = true;
-            n_cur = n_unc;
-            p.rec = (T*)s->rec2; p.hdr = (T*)s->hdr2; p.yrows = (T*)s->yrows2;
-            if (p.tv) p.mdl = (const T*)s->mdl2;
-        }
+        if (5 * n_unc <= 4 * set.n && set.n >= retile_floor)      // a fifth of the tiles to gain: worth the two copies
+            if (set.compact(s, p, n_unc, mdl_per, st)) return -1;
     }
-    if (in_scratch) if (untile_impl<T>(s, n_cur, scratch_map, st)) return -1;
+    if (set.copy_home(s, st)) return -1;
     return 0;
 #else
     (void)s; (void)p; (void)max_iter; (void)check_every; (void)chunked; (void)st;
@@ -582,23 +567,21 @@ static int run_cta_loop(mpcb_solver* s, KParams<T> p, int max_iter, int check_ev
 }
 
 // The ADMM loop on the host side.  The device runs it in chunks of `check_termination` iterations (a chunk ends right
-// after a termination test; unsolved rows stay in p-form, so chunking does not change a single bit).  After a chunk
-// the number of unsolved QPs is read back; once at most half of the current set is left they are RE-TILED — their
-// workspace columns are copied into dense tiles of a scratch workspace — so that warps stop streaming the records of
-// 32 QPs for the sake of one straggler.  At the end the re-tiled QPs are copied back to their home columns.
-// MPCB_NO_RETILE=1 (or "wide" off for a small batch) runs the whole loop as a single asynchronous launch; every other
-// schedule reads the number of unsolved QPs back after each tested launch (a stream synchronisation).
+// after a termination test; unsolved rows stay in p-form, so chunking does not change a single bit).  A batch that shares
+// one KKT matrix runs in admm_dense_kernel, one that the CTA-per-tile kernel serves in run_cta_loop; every other batch below
+// retile_min_batch (and every batch with MPCB_NO_RETILE=1) runs the whole loop as ONE asynchronous launch of
+// admm_tma_kernel.  A larger batch runs phase 1 on the home workspace, then reads the number of unsolved QPs back after
+// each tested launch (a stream synchronisation) and compacts them — their workspace columns are copied into dense tiles
+// of a scratch workspace — every time a fifth of the set has terminated, so that warps stop streaming the records of 32
+// QPs for the sake of one straggler; the tail finishes in the CTA-per-tile kernel.  At the end the compacted QPs are
+// copied back to their home columns.
 template <typename T, typename L>
 static int run_admm_impl(mpcb_solver* s, int max_iter, int check_every, int warm, rt_stream st) {
     const bool no_retile = g_opt_retile.load() == 0;
     const int retile_min = g_opt_retile_min.load();
     const int B = s->batch;
     if (s->cold_pending) { warm = 0; s->cold_pending = false; }      // first launch after prob.setup(): x = z = y = 0
-    // time-varying sets up to 16384 QPs run their steady-state iterations with 8 lanes per QP (see launch_wide) — when
-    // that kernel covers the shape (nx + nu <= 8); otherwise they are chunked and re-tiled like everything else
-    const bool tv_wide = s->prob.time_varying && B <= 16384 && g_opt_wide.load() != 0 &&
-                         s->prob.nx + s->prob.nu <= WIDE_G_HOST;
-    const bool chunked = !no_retile && check_every > 0 && check_every < max_iter && B >= retile_min && !tv_wide;
+    const bool chunked = !no_retile && check_every > 0 && check_every < max_iter && B >= retile_min;
     int* status = s->status;
     if (int r = launch_1d(B, st, MPCB_LAMBDA(int b) { status[b] = status[b] == -7 ? -7 : (int)kUnsolved; })) return r;
     if (int r = rt_memset(s->n_surv, 0, sizeof(int), st)) return r;
@@ -609,7 +592,10 @@ static int run_admm_impl(mpcb_solver* s, int max_iter, int check_every, int warm
     // in one launch — first iteration, termination tests, certificates, exit pass — with the stage models staged by TMA
     // A batch that shares ONE KKT matrix (one linearisation and identical scalings, or a batch of one): the whole loop as a
     // dense GEMM on the FP64 tensor cores in one launch, termination tests included — nothing to read back (admm_dense.cuh)
-    if (!chunked && !no_retile && check_every > 1 && check_every < max_iter) {
+    // (also offered to time-varying batches of up to 16384 QPs with nx + nu <= 8: moved to another kernel, their results
+    // would change in the last bits)
+    const bool dense_window = B < retile_min || (p.tv && B <= 16384 && L::NW <= 8);
+    if (dense_window && !no_retile && check_every > 1 && check_every < max_iter) {
         if (s->dense_state == 0 && dense_candidate<T, L>(s))
             if (int r = ensure_factor_form<T, L>(s, p, false, st)) return r;      // (reads Linv)
         if (int r = dense_prepare<T, L>(s, st)) return r;
@@ -630,26 +616,17 @@ static int run_admm_impl(mpcb_solver* s, int max_iter, int check_every, int warm
         const int rc = run_cta_loop<T, L>(s, p, max_iter, check_every, cta_chunked, st);
         if (rc <= 0) return rc < 0 ? (int)MPCB_E_CUDA : 0;
     }
-    // Small batches (and time-varying sets, see launch_wide) are latency-bound from the first iteration on — a few warps
-    // of the main kernel, each walking 42 dependent stage sweeps per iteration: when the 8-lanes-per-QP kernel covers
-    // the shape it runs every iteration between termination tests (all_wide); iteration 1 (rows enter as explicit
-    // (z, y)) and the tested iterations go through the main kernel.
-    bool all_wide = !chunked && !no_retile && check_every > 1 && check_every < max_iter;
-    if (all_wide) all_wide = L::NW <= WIDE_G_HOST && g_opt_wide.load() != 0;
-    if (!chunked && !all_wide) {
+    if (!chunked) {
         p.it0 = 0; p.it_stop = max_iter; p.list_survivors = 0;
         return launch_admm<T, L>(p, s, st);
     }
     // Large batches: phase 1 on the home workspace up to the iteration count at which the previous solve of this
-    // solver re-tiled (one launch; unknown on the first solve: explore check by check).  Either way the unsolved
-    // count is read after every tested launch; once at most half of the set is left it is re-tiled into dense
-    // tiles of the scratch workspace, where the stragglers finish (8 lanes per QP while the set is small enough).
+    // solver compacted (one launch; unknown on the first solve: explore check by check), then compaction (below).
     // (cold and warm-started solves of one solver converge very differently — the closed loop's step 0 against every later
     // step — so each keeps its own learnt point)
     const int rt_slot = warm ? 1 : 0;
-    int it0 = 0, n_cur = B, which = 0;
-    bool in_scratch = false;
-    const int* scratch_map = nullptr;
+    int it0 = 0;
+    LoopSet<T, L> set{B};
     const bool trace = std::getenv("MPCB_TRACE") != nullptr;
     const auto t_start = std::chrono::steady_clock::now();
     auto trace_ms = [&]() {            // (MPCB_TRACE only) drains the stream: a timestamp per launch, not a product path
@@ -659,31 +636,11 @@ static int run_admm_impl(mpcb_solver* s, int max_iter, int check_every, int warm
     bool learnt_now = false;
     while (it0 < max_iter) {
         int stop = it0 + check_every;
-        if (in_scratch && all_wide) stop = max_iter;
-        else if (it0 == 0 && s->retile_at[rt_slot] > 0 && !all_wide) stop = s->retile_at[rt_slot];
-        p.B = n_cur; p.survivors = s->surv[which]; p.qp_map = in_scratch ? scratch_map : nullptr;
-        if (in_scratch || all_wide) {
-            // The iterations before the next termination test run with 8 lanes per QP (the last of them also saves
-            // the old state), the tested one in the main kernel.
-            int next_test = (it0 / check_every + 1) * check_every;
-            if (next_test > max_iter) next_test = max_iter;
-            if (all_wide) stop = next_test;
-            if (it0 == 0 && next_test > 1) {          // iteration 1 alone (only reached with all_wide)
-                p.it0 = 0; p.it_stop = 1; p.list_survivors = 0;
-                if (int r = launch_admm<T, L>(p, s, st)) return r;
-                it0 = 1;
-            }
-            if (next_test - 1 > it0) {
-                p.it0 = it0; p.it_stop = next_test - 1;
-                const int rw = launch_wide<T, L>(p, st);
-                if (rw < 0) return (int)MPCB_E_CUDA;
-                if (trace) std::fprintf(stderr, "[mpcb] wide %d..%d n=%d -> %d  t=%.3f ms\n", p.it0 + 1, p.it_stop, n_cur, rw, trace_ms());
-                if (rw == 0) { it0 = next_test - 1; stop = next_test; }
-            }
-        }
+        if (it0 == 0 && s->retile_at[rt_slot] > 0) stop = s->retile_at[rt_slot];
+        p.B = set.n; p.survivors = s->surv[set.which]; p.qp_map = set.map;
         p.it0 = it0; p.it_stop = stop < max_iter ? stop : max_iter; p.list_survivors = 1;
         if (int r = launch_admm<T, L>(p, s, st)) return r;
-        if (trace) std::fprintf(stderr, "[mpcb] admm %d..%d n=%d scratch=%d  t=%.3f ms\n", p.it0 + 1, p.it_stop, n_cur, (int)in_scratch, trace_ms());
+        if (trace) std::fprintf(stderr, "[mpcb] admm %d..%d n=%d scratch=%d  t=%.3f ms\n", p.it0 + 1, p.it_stop, set.n, (int)(set.map != nullptr), trace_ms());
         it0 = p.it_stop;
         int n_unc = 0;
         if (int r = rt_d2h(&n_unc, s->n_surv, sizeof(int), st)) return r;
@@ -693,7 +650,7 @@ static int run_admm_impl(mpcb_solver* s, int max_iter, int check_every, int warm
             // Everything terminated where nothing had been compacted: the next solve of this kind runs up to here in one launch
             // — and, once in a while, stops one test earlier to see whether a compaction there pays (a warm-started closed
             // loop drifts from "all at 50" to "half at 25, half at 50" as the scenarios settle).
-            if (!all_wide && !in_scratch && !learnt_now && n_unc == 0) {
+            if (!set.map && !learnt_now && n_unc == 0) {
                 int& at = s->retile_at[rt_slot];
                 int& backoff = s->retile_backoff[rt_slot];
                 if (at == it0 && it0 > check_every && backoff == 0) at = it0 - check_every;
@@ -705,54 +662,40 @@ static int run_admm_impl(mpcb_solver* s, int max_iter, int check_every, int warm
         // Compaction.  Copying a QP's records into a dense tile (and its iterates back later) costs about the traffic of 1.5
         // iterations of that QP; a tile streams the records of all 32 slots as long as one of them is unsolved.  So a large
         // batch is compacted every time a fifth of the set has terminated (the warm-started closed loop loses 30-50 % of its
-        // QPs at the first test, a cold batch 96 % at the third), always from the home workspace, and as soon as the
-        // unsolved set fits one wave of CTAs it finishes in the CTA-per-tile kernel (below).  Small sets handled by the
-        // 8-lanes kernel (all_wide) are latency-bound up to ~2400 QPs and compacted once, when half is left.
+        // QPs at the first test, a cold batch 96 % at the third), and as soon as the unsolved set fits one wave of CTAs it
+        // finishes in the CTA-per-tile kernel (below).
         // (Measured against it: compacting the cold headline batch already at iteration 50, where 13 % have terminated —
         //  27.5 instead of 25.0 ms per step: a launch boundary costs the warp-per-tile kernel a partly filled last wave,
         //  ~2 ms at this size, more than the 1 ms of traffic the compaction saves.)
 #ifndef MPCB_EMU
-        const bool tail_cta = !p.tv && !all_wide && cta_planned<T, L>(s, n_unc, false, check_every) && cta_applicable<T, L>(s, p);
+        const bool tail_cta = !p.tv && cta_planned<T, L>(s, n_unc, false, check_every) && cta_applicable<T, L>(s, p);
 #else
         const bool tail_cta = false;
 #endif
-        const bool compact = all_wide ? (!in_scratch && 2 * n_unc <= n_cur && n_cur > 2400)
-                                      : (tail_cta || (5 * n_unc <= 4 * n_cur && n_cur >= (retile_min < 1024 ? retile_min : 1024)));
-        if (compact) {
-            if (!all_wide && !learnt_now) { s->retile_at[rt_slot] = it0; learnt_now = true; }
-            if (in_scratch) if (int r = untile_impl<T>(s, n_cur, scratch_map, st)) return r;
-            // re-tile: survivors (listed by QP index = home slot) -> dense tiles of the scratch workspace
-            if (int r = ensure_scratch(s, n_unc, 0)) return r;
-            if (int r = retile_impl<T>(s, n_unc, s->surv[which], st)) return r;
-            scratch_map = s->surv[which];
-            which ^= 1;                       // the next launch lists its survivors in the other buffer
-            in_scratch = true;
-            n_cur = n_unc;
-            p.rec = (T*)s->rec2; p.hdr = (T*)s->hdr2; p.yrows = (T*)s->yrows2;
+        if (tail_cta || (5 * n_unc <= 4 * set.n && set.n >= (retile_min < 1024 ? retile_min : 1024))) {
+            if (!learnt_now) { s->retile_at[rt_slot] = it0; learnt_now = true; }
+            if (int r = set.compact(s, p, n_unc, 0, st)) return r;
 #ifndef MPCB_EMU
             // The stragglers of a large batch are a small batch: when they fit one wave of CTAs they finish in the CTA-per-tile
-            // kernel, all remaining iterations, tests and exits in ONE launch (41 us per iteration against 57 us of the
-            // 8-lanes kernel plus a launch of the main kernel and a read-back per test).  It multiplies with the block
-            // inverse: the factor blocks of the re-tiled copies are converted in place.
+            // kernel, all remaining iterations, tests and exits in ONE launch (41 us per iteration, nothing read back per
+            // test).  It multiplies with the block inverse: the factor blocks of the compacted copies are converted in place.
             if (tail_cta) {
-                if (int r = launch_1d(n_cur * (p.N + 1), st, MinvFromLinvFn<T, L>{p.rec, p.N + 1, n_cur})) return r;
+                if (int r = launch_1d(set.n * (p.N + 1), st, MinvFromLinvFn<T, L>{p.rec, p.N + 1, set.n})) return r;
                 KParams<T> pc = p;
-                pc.minv = 1; pc.B = n_cur; pc.qp_map = scratch_map; pc.survivors = s->surv[which];
+                pc.minv = 1; pc.B = set.n; pc.qp_map = set.map; pc.survivors = s->surv[set.which];
                 pc.it0 = it0; pc.it_stop = max_iter; pc.list_survivors = 0;
                 const int rc = launch_cta<T, L>(pc, s, st);
                 if (rc < 0) return (int)MPCB_E_CUDA;
-                if (trace) std::fprintf(stderr, "[mpcb] cta %d..%d n=%d scratch=1 (stragglers)  t=%.3f ms\n", it0 + 1, max_iter, n_cur, trace_ms());
+                if (trace) std::fprintf(stderr, "[mpcb] cta %d..%d n=%d scratch=1 (stragglers)  t=%.3f ms\n", it0 + 1, max_iter, set.n, trace_ms());
                 if (rc == 0) break;
             }
 #endif
-        } else if (!in_scratch && !all_wide && !learnt_now && it0 == s->retile_at[rt_slot]) {
+        } else if (!set.map && !learnt_now && it0 == s->retile_at[rt_slot]) {
             s->retile_at[rt_slot] = 0;                 // the learnt point no longer fits this workload: explore again next time
             s->retile_backoff[rt_slot] = 16;           // (and leave earlier probes alone for a while)
         }
     }
-    if (in_scratch)
-        if (int r = untile_impl<T>(s, n_cur, scratch_map, st)) return r;
-    return 0;
+    return set.copy_home(s, st);
 }
 
 // =============================================================================================

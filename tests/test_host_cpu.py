@@ -59,7 +59,7 @@ def test_long_horizon_time_varying_dynamics(emu_backend):
     pc.check_dynamic_long_horizon(emu_backend, B=2, N=30)
 
 
-def test_retiling_is_bitwise_neutral(emu_backend):
+def test_retiling_is_bitwise_neutral_and_stragglers_match_oracle(emu_backend):
     pc.check_retiling_is_bitwise_neutral(emu_backend, B=40)
 
 
