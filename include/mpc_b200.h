@@ -183,10 +183,14 @@ int mpcb_to_element_major(int dtype, int batch, int elems, size_t ld, const void
 int mpcb_to_batch_major(int dtype, int batch, int elems, size_t ld, const void* src, void* dst_rowmajor, void* stream);
 
 /* Process-wide tunables (also read once from the environment: MPCB_NO_TMA, MPCB_NO_RETILE, MPCB_RETILE_MIN_BATCH,
- * MPCB_NO_CERT, MPCB_NO_DENSE, MPCB_NO_CTA, MPCB_NO_WARP_SETUP):
+ * MPCB_NO_CERT, MPCB_NO_DENSE, MPCB_NO_CTA, MPCB_NO_WARP_SETUP, MPCB_NO_FWD_RHS):
  *   "tma"              1 (default) warp-per-tile ADMM kernel with TMA-staged stage records; 0: one lane per QP from global memory
  *   "retile"           1 (default) run the ADMM loop in chunks and re-tile unconverged QPs; 0: one asynchronous launch
  *   "retile_min_batch" smallest batch that is run in chunks (default 4096)
+ *   "fwd_rhs"          1 (default) the forward sweeps of the warp-per-tile and lane-per-QP kernels after the first iteration
+ *                      of a solve start from the local right-hand side each backward sweep leaves in the stage record and
+ *                      read 43 instead of 65 elements of a configs[2] record; 0: they form the whole right-hand side from
+ *                      the record (the same arithmetic in another order: results agree to rounding)
  *   "dense"            1 (default) a batch that shares ONE KKT matrix (shared_model, identical Ruiz scaling of every QP, f64,
  *                      (N+1)(nx+nu) <= 128) runs its steady-state iterations as a dense FP64 tensor-core GEMM with the
  *                      explicit inverse of the reduced KKT matrix (admm_dense.cuh); 0: the per-QP kernels

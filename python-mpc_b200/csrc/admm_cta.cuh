@@ -122,7 +122,8 @@ __global__ void __launch_bounds__(L::NW * 32, NBUF == CTA_NBUF ? 2 : 1) admm_cta
     typedef CtaSmem<T, L, TV, NBUF> SM;
     typedef CtaModel<L> CM;
     constexpr int RS = SM::RS;
-    constexpr unsigned REC_BYTES = L::REC * TILE * sizeof(T), FWD_BYTES = L::REC_FWD * TILE * sizeof(T),
+    // the forward sweep forms its whole right-hand side: it loads all of a record but the t slots (two runs)
+    constexpr unsigned REC_BYTES = L::REC * TILE * sizeof(T), FWD_BYTES = (L::REC - L::NW) * TILE * sizeof(T),
                        MDL_BYTES = CM::M_XR * TILE * sizeof(T), XR_BYTES = L::NX * TILE * sizeof(T);
     extern __shared__ __align__(128) unsigned char smem_raw[];
     T* const bufs = reinterpret_cast<T*>(smem_raw);
@@ -211,12 +212,12 @@ __global__ void __launch_bounds__(L::NW * 32, NBUF == CTA_NBUF ? 2 : 1) admm_cta
     bool active = valid;
     int status = kUnsolved, it_done = 0;
 
-    // Loop-invariant record offsets of this warp's component.  Variables of a stage are laid out x | slack | u and the bound
+    // Loop-invariant record offsets of this warp's component.  Variables of a stage are laid out slack | x | u and the bound
     // rows bx | bu are contiguous, so component a — a state or an input — finds its scaling, iterate and bound row at one
     // run-time offset each: the x warps and the u warps run the SAME instructions (an input is a state without dynamics
     // rows, cost-reference and slack: its E_dyn, Q and W factors are zero), which is what keeps the stage at ~200
     // instructions per warp — the chain of a stage is bound by issue latency, not by the FP64 pipe.
-    static_assert(L::OBU == L::OBX + NX && L::OX == 0, "component a: variable a (+NS for inputs), bound row OBX + a");
+    static_assert(L::OBU == L::OBX + NX && L::OU == L::OX + NX, "component a: variable OX + a, bound row OBX + a");
     const int cv = isx ? L::OX + jx : L::OU + ju;           // my variable inside D / x
     constexpr int RB = L::OBX;                              // my bound row: RB + a
     const int4* const mrow = reinterpret_cast<const int4*>(mtab + a * MTW);
@@ -231,7 +232,13 @@ __global__ void __launch_bounds__(L::NW * 32, NBUF == CTA_NBUF ? 2 : 1) admm_cta
             T* dst = bufs + (size_t)bi * (RS * TILE);
             const unsigned rb = fwd ? FWD_BYTES : REC_BYTES;
             mbar_expect_tx(br, rb + (TV ? MDL_BYTES : 0u) + ((TV && fwd) ? XR_BYTES : 0u));
-            tma_load_1d(dst, rec_tile + (size_t)k * L::REC * TILE, rb, br);
+            const T* src = rec_tile + (size_t)k * L::REC * TILE;
+            if (fwd) {
+                tma_load_1d(dst, src, L::R_T * TILE * sizeof(T), br);
+                tma_load_1d(dst + L::R_P * TILE, src + L::R_P * TILE, (L::REC - L::R_P) * TILE * sizeof(T), br);
+            } else {
+                tma_load_1d(dst, src, rb, br);
+            }
             if (TV) tma_load_1d(dst + L::REC * TILE, mdl_tile + (size_t)k * CM::COUNT * TILE, MDL_BYTES, br);
             if (TV && fwd) tma_load_1d(dst + L::R_T * TILE, mdl_tile + ((size_t)k * CM::COUNT + CM::M_XR) * TILE, XR_BYTES, br);
         }
@@ -285,7 +292,8 @@ __global__ void __launch_bounds__(L::NW * 32, NBUF == CTA_NBUF ? 2 : 1) admm_cta
             if (wr) {
                 for (int k = a; k <= N; k += NW) {
                     const T* R = ws.R(k); T* O = ws.S(k);
-                    for (int e = 0; e < L::VS + L::CS; ++e) MPCB_AT(O, e) = MPCB_AT(R, L::R_X + e);
+                    for (int e = 0; e < L::VS; ++e) MPCB_AT(O, e) = MPCB_AT(R, L::R_X + e);
+                    for (int e = 0; e < L::CS; ++e) MPCB_AT(O, L::VS + e) = MPCB_AT(R, L::R_P + e);
                 }
                 if (a == 0)
                     for (int i = 0; i < NX; ++i) MPCB_AT(ws.scr_hdr, i) = MPCB_AT(ws.hdr, L::H_P0 + i);

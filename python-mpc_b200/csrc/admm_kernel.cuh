@@ -56,9 +56,11 @@ void admm_save_old_raw(const T* rec, T* scr, const T* hdr, T* scr_hdr, int N) {
     for (int k = 0; k <= N; ++k) {
         const T* R = rec + (size_t)k * L::REC * TILE;
         T* O = scr + (size_t)k * NE * TILE;
-        T tmp[NE];
+        T tmp[NE];       // [x | p], the order of the old-state buffer
 #pragma unroll
-        for (int e = 0; e < NE; ++e) tmp[e] = MPCB_AT(R, L::R_X + e);
+        for (int e = 0; e < L::VS; ++e) tmp[e] = MPCB_AT(R, L::R_X + e);
+#pragma unroll
+        for (int e = 0; e < L::CS; ++e) tmp[L::VS + e] = MPCB_AT(R, L::R_P + e);
 #pragma unroll
         for (int e = 0; e < NE; ++e) MPCB_AT(O, e) = tmp[e];
     }
@@ -191,15 +193,16 @@ MPCB_HD void admm_finish(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T,
 }
 
 // Forward and backward sweep of one iteration straight out of global memory.  FIRST (iteration 1 of a solve: rows
-// enter as explicit (z, y)) and SAVE (the next iteration is tested: duplicate the new state into the old-state buffer)
-// are template parameters: the steady-state instantiation carries none of that code or state.
-template <typename T, typename L, bool FIRST>
+// enter as explicit (z, y)), RHS (the forward sweep starts from r^) and SAVE (the next iteration is tested: duplicate the
+// new state into the old-state buffer) are template parameters: the steady-state instantiation carries none of that code
+// or state.
+template <typename T, typename L, bool FIRST, bool RHS = false>
 MPCB_HD void admm_one_fwd(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T, L>& m, int bi, const Ws<T, L>& ws) {
     FwdCarry<T, L> cy;
     admm_fwd_begin<T, L, FIRST>(p, q, bi, ws.hdr, cy);
     for (int k = 0; k <= p.N; ++k) {
         if (p.tv && k < p.N) load_model<T, L>(p, bi, k, m);
-        admm_fwd_stage<T, L, FIRST>(p, q, m, bi, k, ws.R(k), ws.Y(k), ws.R(k), cy);
+        admm_fwd_stage<T, L, FIRST, RHS>(p, q, m, bi, k, ws.R(k), ws.Y(k), ws.R(k), cy);
     }
 }
 template <typename T, typename L, bool FIRST, bool SAVE>
@@ -239,7 +242,8 @@ MPCB_HD void admm_one(const KParams<T>& p, int b) {
         if (admm_needs_copy(p, it)) admm_save_old_all<T, L>(p, ws);
         if (first) { admm_one_fwd<T, L, true>(p, q, m, bi, ws); admm_one_bwd<T, L, true, false>(p, q, m, bi, ws); }
         else {
-            admm_one_fwd<T, L, false>(p, q, m, bi, ws);
+            if (p.fwd_rhs) admm_one_fwd<T, L, false, true>(p, q, m, bi, ws);
+            else admm_one_fwd<T, L, false>(p, q, m, bi, ws);
             if (admm_saves(p, it)) admm_one_bwd<T, L, false, true>(p, q, m, bi, ws);
             else admm_one_bwd<T, L, false, false>(p, q, m, bi, ws);
         }
@@ -306,17 +310,38 @@ __device__ __forceinline__ void tma_load_1d(void* dst_smem, const void* src_gmem
 // order this thread's generic-proxy writes before later async-proxy (TMA) reads of the same memory
 __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async;" ::: "memory"); }
 
+// What a TMA load of a stage record brings into a record buffer (one mbarrier transaction, one or two bulk copies):
+//   kLoadAll  the whole record: the backward sweep, and stage 0 / stage N of a forward sweep (the backward turn-around)
+//   kLoadFwd  all but t: a forward sweep that forms the whole right-hand side, and the termination sweep
+//   kLoadRhs  the runs FA and FB: a forward sweep that starts from r^ (mpc_common.h)
+enum { kLoadAll, kLoadFwd, kLoadRhs };
+template <typename T, typename L, int WHAT>
+__device__ __forceinline__ void tma_load_stage(T* dst, const T* src, unsigned long long* bar) {
+    constexpr unsigned E = TILE * sizeof(T);
+    if (WHAT == kLoadRhs) {
+        mbar_expect_tx(bar, (L::FA_N + L::FB_N) * E);
+        tma_load_1d(dst + L::FA * TILE, src + L::FA * TILE, L::FA_N * E, bar);
+        tma_load_1d(dst + L::FB * TILE, src + L::FB * TILE, L::FB_N * E, bar);
+    } else if (WHAT == kLoadFwd) {
+        mbar_expect_tx(bar, (L::REC - L::NW) * E);
+        tma_load_1d(dst, src, L::R_T * E, bar);
+        tma_load_1d(dst + L::R_P * TILE, src + L::R_P * TILE, (L::REC - L::R_P) * E, bar);
+    } else {
+        mbar_expect_tx(bar, L::REC * E);
+        tma_load_1d(dst, src, L::REC * E, bar);
+    }
+}
+
 // Forward and backward sweep of one iteration of a tile: record k is resident in one of the warp's two buffers while
 // the elected lane has the TMA bulk load of the next record in flight into the other.  FIRST = iteration 1 of a solve
-// (rows enter as explicit (z, y)), SAVE = the next iteration is tested (the new state is duplicated into the old-state
-// buffer); the steady-state instantiation carries none of that code or state.
-template <typename T, typename L, bool FIRST>
+// (rows enter as explicit (z, y)), RHS = the forward sweep starts from r^ and loads only the runs FA and FB of the
+// records in between, SAVE = the next iteration is tested (the new state is duplicated into the old-state buffer); the
+// steady-state instantiation carries none of that code or state.  Record 0 of a forward sweep is resident whole (the
+// backward turn-around patches it, or a kLoadAll), so is record N (loaded whole for the backward turn-around).
+template <typename T, typename L, bool FIRST, bool RHS>
 __device__ __forceinline__ void admm_tma_fwd(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T, L>& m,
                                              const Ws<T, L>& ws, int bb, int lane, bool active, T* buf0,
                                              unsigned long long* bar, unsigned& ph, int& cur, const T* rec_tile) {
-    constexpr unsigned REC_BYTES = L::REC * TILE * sizeof(T);
-    constexpr unsigned FWD_BYTES = L::REC_FWD * TILE * sizeof(T);
-    (void)REC_BYTES; (void)FWD_BYTES;
     const int N = p.N;
 #define MPCB_BUF(c) (buf0 + (c) * (L::REC * TILE))
     // ---------------- forward sweep: record k is resident in MPCB_BUF(cur); prefetch k+1
@@ -325,13 +350,14 @@ __device__ __forceinline__ void admm_tma_fwd(const KParams<T>& p, const AdmmCons
         admm_fwd_begin<T, L, FIRST>(p, q, bb, ws.hdr, cy);
         for (int k = 0; k <= N; ++k) {
             if (k < N && lane == 0) {
-                mbar_expect_tx(&bar[cur ^ 1], FWD_BYTES);
-                tma_load_1d(MPCB_BUF(cur ^ 1), rec_tile + (size_t)(k + 1) * L::REC * TILE, FWD_BYTES, &bar[cur ^ 1]);
+                const T* src = rec_tile + (size_t)(k + 1) * L::REC * TILE;
+                if (k + 1 == N) tma_load_stage<T, L, kLoadAll>(MPCB_BUF(cur ^ 1), src, &bar[cur ^ 1]);
+                else tma_load_stage<T, L, RHS ? kLoadRhs : kLoadFwd>(MPCB_BUF(cur ^ 1), src, &bar[cur ^ 1]);
             }
             if (k > 0) { mbar_wait(&bar[cur], (ph >> cur) & 1u); ph ^= 1u << cur; }
             if (active) {
                 if (p.tv && k < N) load_model<T, L>(p, bb, k, m);
-                admm_fwd_stage<T, L, FIRST>(p, q, m, bb, k, MPCB_BUF(cur) + lane, ws.Y(k), ws.R(k), cy);
+                admm_fwd_stage<T, L, FIRST, RHS>(p, q, m, bb, k, MPCB_BUF(cur) + lane, ws.Y(k), ws.R(k), cy);
                 if (k == N) {                     // turn-around: backward stage N reuses this buffer, give it t_N
 #pragma unroll
                     for (int a = 0; a < L::NW; ++a)
@@ -349,9 +375,6 @@ template <typename T, typename L, bool FIRST, bool SAVE>
 __device__ __forceinline__ void admm_tma_bwd(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T, L>& m,
                                              const Ws<T, L>& ws, int bb, int lane, bool active, T* buf0,
                                              unsigned long long* bar, unsigned& ph, int& cur, const T* rec_tile) {
-    constexpr unsigned REC_BYTES = L::REC * TILE * sizeof(T);
-    constexpr unsigned FWD_BYTES = L::REC_FWD * TILE * sizeof(T);
-    (void)REC_BYTES; (void)FWD_BYTES;
     const int N = p.N;
 #define MPCB_BUF(c) (buf0 + (c) * (L::REC * TILE))
     // ---------------- backward sweep: record N is resident in MPCB_BUF(cur); prefetch k-1 (with t)
@@ -360,24 +383,19 @@ __device__ __forceinline__ void admm_tma_bwd(const KParams<T>& p, const AdmmCons
 #pragma unroll
         for (int i = 0; i < L::NX; ++i) { cy.xt_next[i] = 0; cy.Dx_next[i] = 1; }
         for (int k = N; k >= 0; --k) {
-            if (k > 0 && lane == 0) {
-                mbar_expect_tx(&bar[cur ^ 1], REC_BYTES);
-                tma_load_1d(MPCB_BUF(cur ^ 1), rec_tile + (size_t)(k - 1) * L::REC * TILE, REC_BYTES, &bar[cur ^ 1]);
-            }
+            if (k > 0 && lane == 0)
+                tma_load_stage<T, L, kLoadAll>(MPCB_BUF(cur ^ 1), rec_tile + (size_t)(k - 1) * L::REC * TILE, &bar[cur ^ 1]);
             if (k < N) { mbar_wait(&bar[cur], (ph >> cur) & 1u); ph ^= 1u << cur; }
             if (active) {
                 if (p.tv && k < N) load_model<T, L>(p, bb, k, m);
                 admm_bwd_stage<T, L, FIRST, SAVE>(p, q, m, bb, k, MPCB_BUF(cur) + lane, ws.Y(k), ws.R(k), cy, ws.S(k));
-                if (k == 0) {                     // turn-around: the next forward stage 0 reuses this buffer
+                if (k == 0) {                     // turn-around: the next forward stage 0 reuses this buffer: new r^, p, x
 #pragma unroll
-                    for (int e = 0; e < L::VS; ++e)
-                        MPCB_AT(MPCB_BUF(cur) + lane, L::R_X + e) = MPCB_AT(ws.R(0), L::R_X + e);
-#pragma unroll
-                    for (int e = 0; e < L::CS; ++e)
-                        MPCB_AT(MPCB_BUF(cur) + lane, L::R_P + e) = MPCB_AT(ws.R(0), L::R_P + e);
+                    for (int e = 0; e < L::NW + L::CS + L::VS; ++e)
+                        MPCB_AT(MPCB_BUF(cur) + lane, L::R_T + e) = MPCB_AT(ws.R(0), L::R_T + e);
                 }
             }
-            if (k == 0) fence_proxy_async();      // new x, p (generic stores) before the next sweep's TMA reads
+            if (k == 0) fence_proxy_async();      // new r^, x, p (generic stores) before the next sweep's TMA reads
             __syncwarp();
             if (k > 0) cur ^= 1;
         }
@@ -390,7 +408,6 @@ template <typename T, typename L>
 __global__ void __launch_bounds__(256, 1) admm_tma_kernel(const __grid_constant__ KParams<T> p, int* tile_counter) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr unsigned REC_BYTES = L::REC * TILE * sizeof(T);
-    constexpr unsigned FWD_BYTES = L::REC_FWD * TILE * sizeof(T);
     const int warps = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int N = p.N, ntiles = (p.B + TILE - 1) / TILE;
     T* const buf0 = reinterpret_cast<T*>(smem_raw + (size_t)warp * 2 * REC_BYTES);     // two record buffers of this warp
@@ -475,7 +492,7 @@ __global__ void __launch_bounds__(256, 1) admm_tma_kernel(const __grid_constant_
             fence_proxy_async();
             __syncwarp();
             // record 0 for the first forward sweep
-            if (lane == 0) { mbar_expect_tx(&bar[cur], FWD_BYTES); tma_load_1d(MPCB_BUF(cur), rec_tile, FWD_BYTES, &bar[cur]); }
+            if (lane == 0) tma_load_stage<T, L, kLoadAll>(MPCB_BUF(cur), rec_tile, &bar[cur]);
             mbar_wait(&bar[cur], (ph >> cur) & 1u); ph ^= 1u << cur;
         }
 
@@ -496,10 +513,11 @@ __global__ void __launch_bounds__(256, 1) admm_tma_kernel(const __grid_constant_
 #endif
                 // ---------------- forward and backward sweep (the steady-state instantiation has no first-iteration code)
                 if (first) {
-                    admm_tma_fwd<T, L, true>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
+                    admm_tma_fwd<T, L, true, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
                     admm_tma_bwd<T, L, true, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
                 } else {
-                    admm_tma_fwd<T, L, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
+                    if (p.fwd_rhs) admm_tma_fwd<T, L, false, true>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
+                    else admm_tma_fwd<T, L, false, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
 #if MPCB_SAVE_BY_COPY
                     admm_tma_bwd<T, L, false, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
 #else
@@ -523,10 +541,8 @@ __global__ void __launch_bounds__(256, 1) admm_tma_kernel(const __grid_constant_
                     if (open_) admm_test_begin<T, L>(p, q, bb, ws.hdr, cy, t, cert, first, ws.scr_hdr);   // buffer `cur` holds record 0
                     for (int k = 0; k <= N; ++k) {
                         if (k < N) {
-                            if (lane == 0) {
-                                mbar_expect_tx(&bar[cur ^ 1], FWD_BYTES);
-                                tma_load_1d(MPCB_BUF(cur ^ 1), rec_tile + (size_t)(k + 1) * L::REC * TILE, FWD_BYTES, &bar[cur ^ 1]);
-                            }
+                            if (lane == 0)
+                                tma_load_stage<T, L, kLoadFwd>(MPCB_BUF(cur ^ 1), rec_tile + (size_t)(k + 1) * L::REC * TILE, &bar[cur ^ 1]);
                             mbar_wait(&bar[cur ^ 1], (ph >> (cur ^ 1)) & 1u); ph ^= 1u << (cur ^ 1);
                         }
                         if (open_) {
@@ -550,14 +566,14 @@ __global__ void __launch_bounds__(256, 1) admm_tma_kernel(const __grid_constant_
                     }
                     if (cert || !__any_sync(0xffffffffu, open_)) break;
                     // the certificate pass starts again from record 0
-                    if (lane == 0) { mbar_expect_tx(&bar[cur ^ 1], FWD_BYTES); tma_load_1d(MPCB_BUF(cur ^ 1), rec_tile, FWD_BYTES, &bar[cur ^ 1]); }
+                    if (lane == 0) tma_load_stage<T, L, kLoadFwd>(MPCB_BUF(cur ^ 1), rec_tile, &bar[cur ^ 1]);
                     mbar_wait(&bar[cur ^ 1], (ph >> (cur ^ 1)) & 1u); ph ^= 1u << (cur ^ 1);
                     cur ^= 1;
                 }
                 if (!__any_sync(0xffffffffu, active)) alive = false;     // every QP of the tile is done: no more sweeps
                 else {
-                    // the next forward sweep expects record 0 in the current buffer
-                    if (lane == 0) { mbar_expect_tx(&bar[cur ^ 1], FWD_BYTES); tma_load_1d(MPCB_BUF(cur ^ 1), rec_tile, FWD_BYTES, &bar[cur ^ 1]); }
+                    // the next forward sweep expects record 0 (whole, r^ included) in the current buffer
+                    if (lane == 0) tma_load_stage<T, L, kLoadAll>(MPCB_BUF(cur ^ 1), rec_tile, &bar[cur ^ 1]);
                     mbar_wait(&bar[cur ^ 1], (ph >> (cur ^ 1)) & 1u); ph ^= 1u << (cur ^ 1);
                     cur ^= 1;
                 }

@@ -23,6 +23,7 @@ std::atomic<int> g_opt_dense{std::getenv("MPCB_NO_DENSE") ? 0 : 1};
 std::atomic<int> g_opt_cta{std::getenv("MPCB_NO_CTA") ? 0 : 1};
 std::atomic<int> g_opt_warp_setup{std::getenv("MPCB_NO_WARP_SETUP") ? 0 : 1};
 std::atomic<int> g_opt_retile_min{env_int("MPCB_RETILE_MIN_BATCH", 4096)};
+std::atomic<int> g_opt_fwd_rhs{std::getenv("MPCB_NO_FWD_RHS") ? 0 : 1};
 int fail(int code, const std::string& msg) {
     g_err = msg;
     return code;
@@ -82,6 +83,7 @@ int mpcb_set_option(const char* name, int value) {
     else if (n == "warp_setup") g_opt_warp_setup = value != 0;
     else if (n == "cta") g_opt_cta = value < 0 ? 0 : (value > 2 ? 2 : value);
     else if (n == "retile_min_batch") g_opt_retile_min = value;
+    else if (n == "fwd_rhs") g_opt_fwd_rhs = value != 0;
     else return fail(MPCB_E_ARG, "unknown option: " + n);
     return 0;
 }
@@ -299,7 +301,8 @@ template <typename T>
 static int gather_impl(mpcb_solver* s, void* x_out, void* y_out, void* u_out, rt_stream st) {
     const int N = s->prob.horizon, nx = s->prob.nx, nu = s->prob.nu, ns = s->prob.slack ? nx : 0;
     const int VS = s->VS, CS = s->CS, REC = s->REC, nvar = s->nvar, ncon = s->ncon, B = s->batch;
-    const int R_D = 0, R_E = VS, R_X = VS + CS + s->LT, H_E0 = 0, H_Y0 = 2 * nx, H_C = 3 * nx, HDR = s->HDR;
+    // record layout (Lay, mpc_common.h): [ D | E | Linv | t | p | x ], variables s | x | u inside D and x
+    const int R_D = 0, R_E = VS, R_X = VS + CS + s->LT + s->NW + CS, H_E0 = 0, H_Y0 = 2 * nx, H_C = 3 * nx, HDR = s->HDR;
     const size_t S1 = (size_t)(N + 1);
     const T* rec = (const T*)s->rec; const T* hdr = (const T*)s->hdr; const T* yr = (const T*)s->yrows;
     // a QP that ended with an infeasibility certificate has no solution: NaN like OSQP's results (osqp.c: store_solution)
@@ -317,8 +320,8 @@ static int gather_impl(mpcb_solver* s, void* x_out, void* y_out, void* u_out, rt
             const int k = e / VS, o = e - k * VS;
             const T* R = rec + (((size_t)(b >> 5) * S1 + k) * REC) * TILE + (b & 31);
             const T v = MPCB_NO_SOLUTION(b) ? nanv : R[(size_t)(R_D + o) * TILE] * R[(size_t)(R_X + o) * TILE];
-            if (o < nx) { if (xo) xo[(size_t)b * nvar + k * nx + o] = v; }
-            else if (o < nx + ns) { if (xo) xo[(size_t)b * nvar + (N + 1) * nx + N * nu + k * nx + (o - nx)] = v; }
+            if (o < ns) { if (xo) xo[(size_t)b * nvar + (N + 1) * nx + N * nu + k * nx + o] = v; }
+            else if (o < ns + nx) { if (xo) xo[(size_t)b * nvar + k * nx + (o - ns)] = v; }
             else if (k < N) {
                 const int j = o - nx - ns;
                 if (xo) xo[(size_t)b * nvar + (N + 1) * nx + k * nu + j] = v;

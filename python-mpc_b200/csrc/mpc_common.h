@@ -10,13 +10,17 @@
 //   The solver WORKSPACE is tiled: a tile is 32 consecutive QPs (one warp, lane = b % 32).  Per tile
 //   and per stage k there is one contiguous *stage record* of REC elements x 32 lanes
 //       rec[((tile*(N+1) + k)*REC + e)*32 + lane]
-//       e:  [ D (VS) | E (CS) | Linv (LT) | x (VS) | p (CS) | t (NW) ]
+//       e:  [ D (VS) | E (CS) | Linv (LT) | t (NW) | p (CS) | x (VS) ]
 //   holding everything one ADMM sweep needs at that stage: the Ruiz scalings of the stage's
-//   variables [x_k | s_k | u_k] (D) and of the rows the stage OWNS [dyn_{k+1} | bx_k | bu_k] (E), the
-//   inverse Cholesky block Linv_k, the iterates x, the row state p (= z between solves) and the
-//   forward-substitution intermediate t.  Because a record is contiguous (REC*256 bytes in FP64) a
-//   warp stages it into shared memory with ONE cp.async.bulk, and every access inside the record
-//   has a compile-time offset.  A small per-QP header holds the dyn_0 rows (E, p, y) and the cost
+//   variables [s_k | x_k | u_k] (D) and of the rows the stage OWNS [dyn_{k+1} | bx_k | bu_k] (E), the
+//   inverse Cholesky block Linv_k, the t slots, the row state p (= z between solves) and the iterates
+//   x.  The t slots hold the forward-substitution intermediate t between the forward and the backward
+//   sweep, and the stage's local forward right-hand side r^ (written by the backward sweep) between the
+//   backward sweep and the next forward sweep.  Because a record is contiguous (REC*256 bytes in FP64)
+//   a warp stages it into shared memory with ONE cp.async.bulk, and every access inside the record
+//   has a compile-time offset.  The order puts what a forward sweep reads from r^ on in two runs
+//   (FA: D_x | D_u | E_dyn, FB: Linv | r^ | p_dyn), so that it streams 2 NX + NU + LT + NW + NX
+//   elements of the record instead of all but t.  A small per-QP header holds the dyn_0 rows (E, p, y) and the cost
 //   scaling c; the duals y (touched only on entry/exit of a solve) live in a separate tiled array.
 //   (The u / bu slots of stage N and its dyn_{N+1} slot are unused padding.)  The reference's
 //   ordering (x_0..x_N, u_0..u_{N-1}, s_0..s_N) is produced by the gather kernels in mpc_b200.cu.
@@ -84,6 +88,9 @@ struct KParams {
     int certs;        // 1 (default): evaluate OSQP's infeasibility certificates when a residual test fails; 0: statuses
                       //   solved / solved inaccurate / max-iter only (mpcb_set_option("certificates", 0), a diagnostic switch)
     int warm;         // 0: cold start (x = z = y = 0); 1: keep the iterates already in the workspace
+    int fwd_rhs;      // 1 (default): the forward sweeps after the first iteration of a solve start from the local right-hand
+                      //   side r^ the previous backward sweep left in the t slots; 0: every forward sweep forms the whole
+                      //   right-hand side from the record (mpcb_set_option("fwd_rhs", 0))
     // ---- one CHUNK of the ADMM loop (the host runs the loop in chunks so that unconverged QPs can be re-tiled):
     int it0;          // iterations already done; this launch runs it0+1 .. it_stop.  Rows are explicit (z, y) on
     int it_stop;      //   entry when it0 == 0 and stay in p-form across chunk boundaries (bitwise continuation)
@@ -121,11 +128,13 @@ struct Lay {
     static constexpr int CS = 2 * NX_ + NU_;
     static constexpr int LT = NW * (NW + 1) / 2;
     static constexpr int FS = NX_ * NW;
-    static constexpr int OX = 0, OS = NX_, OU = NX_ + NS;      // variables inside a D / x block
+    static constexpr int OS = 0, OX = NS, OU = NS + NX_;       // variables inside a D / x block
     static constexpr int ODN = 0, OBX = NX_, OBU = 2 * NX_;    // rows inside an E / p block: dyn_{k+1}, bx_k, bu_k
-    static constexpr int R_D = 0, R_E = VS, R_F = VS + CS, R_X = R_F + LT, R_P = R_X + VS, R_T = R_P + CS,
-                         REC = R_T + NW;
-    static constexpr int REC_FWD = R_T;                        // the forward sweep does not read t
+    static constexpr int R_D = 0, R_E = VS, R_F = VS + CS, R_T = R_F + LT, R_P = R_T + NW, R_X = R_P + CS,
+                         REC = R_X + VS;
+    // the two runs a forward sweep that starts from r^ reads: FA = D_x | D_u | E_dyn, FB = Linv | r^ | p_dyn
+    static constexpr int FA = R_D + OX, FA_N = R_E + ODN + NX_ - FA;
+    static constexpr int FB = R_F, FB_N = R_P + ODN + NX_ - FB;
     static constexpr int H_E0 = 0, H_P0 = NX_, H_Y0 = 2 * NX_, H_C = 3 * NX_, HDR = 3 * NX_ + 1;
     static MPCB_HD int nvar(int N) { return (N + 1) * NX + N * NU + (N + 1) * NS; }
     static MPCB_HD int ncon(int N) { return 2 * (N + 1) * NX + N * NU; }

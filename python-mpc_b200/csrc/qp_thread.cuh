@@ -564,10 +564,14 @@ struct FwdCarry {
     T cprev[L::NX];      // [A_{k-1} B_{k-1}] (D (.) Linv_{k-1}' t_{k-1})
 };
 
-template <typename T, typename L, bool FIRST>
+// RHS: the right-hand side is r^ (read from the t slots, written by the previous backward sweep) plus the two terms that come
+// from stage k-1; the stage reads only the runs FA and FB of its record (mpc_common.h).  Otherwise it is formed from the
+// whole record (the first iteration of a solve, or with KParams::fwd_rhs = 0).
+template <typename T, typename L, bool FIRST, bool RHS = false>
 MPCB_HD void admm_fwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const Model<T, L>& m, int b, int k,
                             const T* S, const T* Yk, T* R, FwdCarry<T, L>& cy) {
     constexpr bool first = FIRST;     // compile-time: the steady-state sweeps carry no trace of the (z, y) entry form
+    static_assert(!(FIRST && RHS), "r^ is formed from p-form rows: there is none before the first backward sweep");
     constexpr int NX = L::NX, NU = L::NU, NW = L::NW, NS = L::NS;
     const bool last = (k == p.N);
     const T* Qk = last ? p.QN : p.Q;
@@ -588,6 +592,20 @@ MPCB_HD void admm_fwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
         }
         wv[i] = Ed_next[i] * vd_next[i];
     }
+    if (RHS) {
+#pragma unroll
+        for (int j = 0; j < NX; ++j) {
+            const T ex = cy.Ed_cur[j] * Dx[j];
+            T v = MPCB_AT(S, L::R_T + j) - ex * cy.vd_cur[j];
+            if (k > 0) v += q.rho_eq * ex * cy.Ed_cur[j] * cy.cprev[j];
+            r[j] = v;
+        }
+#pragma unroll
+        for (int j = 0; j < NU; ++j) {
+            Du[j] = last ? (T)1 : MPCB_AT(S, L::R_D + L::OU + j);
+            r[NX + j] = MPCB_AT(S, L::R_T + NX + j);
+        }
+    } else {
 #pragma unroll
     for (int j = 0; j < NX; ++j) {
         const T Ebx = MPCB_AT(S, L::R_E + L::OBX + j);
@@ -632,6 +650,8 @@ MPCB_HD void admm_fwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
         }
         r[NX + j] = v;
     }
+    }
+    (void)wv;
     // t = Linv r ;  g = Linv' t ;  h = D (.) g ;  cprev = [A B] h
     T Li[L::LT], t[NW], h[NW];
 #pragma unroll
@@ -675,6 +695,9 @@ struct BwdCarry {
 
 // SAVE: the next iteration ends with a termination test — the new x and row state also go to the old-state buffer O
 // (what the infeasibility certificates of that iteration call x^{k-1}, y^{k-1}); duplicate stores, nothing else.
+// Every instantiation leaves r^_k in the t slots of R: the part of the next forward sweep's right-hand side r_k that depends
+// on stage k alone (sigma x, the cost term, the bound rows and the slack elimination, A'w / B'w of rows dyn_{k+1}), formed
+// from the new x_k and the new p-form rows — all in registers here, while the next forward sweep would have to read them.
 template <typename T, typename L, bool FIRST, bool SAVE>
 MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const Model<T, L>& m, int b, int k,
                             const T* S, const T* Yk, T* R, BwdCarry<T, L>& cy, T* O) {
@@ -723,6 +746,7 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
         w[d] = acc;
     }
     // rows bx_k (+ slack recovery), x_k / s_k
+    T rh[NW];         // r^_k
 #pragma unroll
     for (int j = 0; j < NX; ++j) {
         const T Ebx = MPCB_AT(S, L::R_E + L::OBX + j);
@@ -730,16 +754,17 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
         const T rb = row_rho(q.inf_bounds, lb, ub, q.rho, q.rho_eq);
         const Row<T> rw = row_state_b(first, MPCB_AT(S, L::R_P + L::OBX + j), Yk + (L::OBX + j) * TILE, lb, ub, rb, q);
         T ztil = bx * w[j];
+        T sn = 0, bs = 0, mxs = 0, mss = 1;
         if (NS) {
             const T Dsl = MPCB_AT(S, L::R_D + L::OS + (NS ? j : 0));
-            const T bs = p.S[j] * Ebx * Dsl;
-            const T mss = q.c * p.W[j] * Dsl * Dsl + q.sigma + rb * bs * bs;
-            const T mxs = rb * bx * bs;
+            bs = p.S[j] * Ebx * Dsl;
+            mss = q.c * p.W[j] * Dsl * Dsl + q.sigma + rb * bs * bs;
+            mxs = rb * bx * bs;
             const T sold = MPCB_AT(S, L::R_X + L::OS + (NS ? j : 0));
             const T rs = q.sigma * sold + bs * (rb * (rw.z - rw.yr));
             const T st = (rs - mxs * w[j]) * fast_rcp(mss);
             ztil += bs * st;
-            const T sn = q.alpha * st + ((T)1 - q.alpha) * sold;
+            sn = q.alpha * st + ((T)1 - q.alpha) * sold;
             MPCB_AT(R, L::R_X + L::OS + (NS ? j : 0)) = sn;
             if (SAVE) MPCB_AT(O, L::OS + (NS ? j : 0)) = sn;
         }
@@ -748,7 +773,17 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
         MPCB_AT(R, L::R_P + L::OBX + j) = pn;
         MPCB_AT(R, L::R_X + L::OX + j) = xn;
         if (SAVE) { MPCB_AT(O, L::VS + L::OBX + j) = pn; MPCB_AT(O, L::OX + j) = xn; }
+        // r^: sigma x - q + bx' (rho (z - y/rho)) of the new state, minus the slack elimination (A'w of rows dyn_{k+1} below)
+        const Row<T> rn = row_state(false, pn, (T)0, lb, ub, (T)0);
+        const T vbx = rb * (rn.z - rn.yr);
+        const T xr = p.xr_tv ? p.Xr[((size_t)k * NX + j) * p.ld + b] : q.xr[(size_t)j * q.xr_stride];
+        const T qh = q.c * Dx[j] * (-((last ? p.QN : p.Q)[j] * xr));
+        T v = q.sigma * xn - qh + bx * vbx;
+        if (NS) v -= mxs * fast_rcp(mss) * (q.sigma * sn + bs * vbx);
+        rh[j] = v;
     }
+#pragma unroll
+    for (int j = 0; j < NU; ++j) rh[NX + j] = 0;
     if (!last) {
 #pragma unroll
         for (int j = 0; j < NU; ++j) {
@@ -761,8 +796,11 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
             MPCB_AT(R, L::R_P + L::OBU + j) = pn;
             MPCB_AT(R, L::R_X + L::OU + j) = un;
             if (SAVE) { MPCB_AT(O, L::VS + L::OBU + j) = pn; MPCB_AT(O, L::OU + j) = un; }
+            const Row<T> rn = row_state(false, pn, (T)0, lb, ub, (T)0);
+            rh[NX + j] = q.sigma * un + bu * (rb * (rn.z - rn.yr));
         }
         // rows dyn_{k+1}:  E (A D x~_k + B D u~_k) - ex_{k+1} x~_{k+1} = -E g_k
+        T wv[NX];     // E (rho z - y) of the new rows dyn_{k+1}
 #pragma unroll
         for (int i = 0; i < NX; ++i) {
             T acc = 0;
@@ -777,8 +815,26 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
             const T pn = row_next(ztil, rw, q.alpha);
             MPCB_AT(R, L::R_P + L::ODN + i) = pn;
             if (SAVE) MPCB_AT(O, L::VS + L::ODN + i) = pn;
+            const Row<T> rn = row_state(false, pn, (T)0, beq, beq, (T)0);
+            wv[i] = Ed_next[i] * (q.rho_eq * (rn.z - rn.yr));
+        }
+#pragma unroll
+        for (int j = 0; j < NX; ++j) {
+            T acc = 0;
+#pragma unroll
+            for (int i = 0; i < NX; ++i) acc += m.A[i][j] * wv[i];
+            rh[j] += Dx[j] * acc;
+        }
+#pragma unroll
+        for (int j = 0; j < NU; ++j) {
+            T acc = 0;
+#pragma unroll
+            for (int i = 0; i < NX; ++i) acc += m.B[i][j] * wv[i];
+            rh[NX + j] += Du[j] * acc;
         }
     }
+#pragma unroll
+    for (int a = 0; a < NW; ++a) MPCB_AT(R, L::R_T + a) = rh[a];
 #pragma unroll
     for (int i = 0; i < NX; ++i) { cy.xt_next[i] = w[i]; cy.Dx_next[i] = Dx[i]; }
 }

@@ -22,7 +22,7 @@ using namespace mpcb;
 // compiled (shape, dtype) plus the ABI layer — see __graft_entry__.build_cuda)
 namespace mpcb_rt {
 extern std::atomic<long long> g_launches;
-extern std::atomic<int> g_opt_tma, g_opt_retile, g_opt_cert, g_opt_dense, g_opt_cta, g_opt_warp_setup, g_opt_retile_min;
+extern std::atomic<int> g_opt_tma, g_opt_retile, g_opt_cert, g_opt_dense, g_opt_cta, g_opt_warp_setup, g_opt_retile_min, g_opt_fwd_rhs;
 int fail(int code, const std::string& msg);      // records the message for mpcb_last_error(), returns `code`
 }
 struct ShapeOps;
@@ -174,6 +174,7 @@ static KParams<T> make_params(const mpcb_solver* s) {
     p.xbox = (const T*)s->xbox;
     p.inf_bounds = s->inf_bounds;
     p.certs = g_opt_cert.load();
+    p.fwd_rhs = g_opt_fwd_rhs.load();
     const mpcb_settings& o = s->set;
     p.rho_c = (T)o.rho < (T)kRhoMin ? (T)kRhoMin : ((T)o.rho > (T)kRhoMax ? (T)kRhoMax : (T)o.rho);
     p.rho_eq_c = (T)kRhoEqOverRhoIneq * p.rho_c;

@@ -432,12 +432,13 @@ static int retile_impl(mpcb_solver* s, int n, const int* list, rt_stream st) {
         else { const size_t h = (size_t)e - S1 * REC; hdr2[(td * HDR + h) * TILE + ldn] = hdr[(ts * HDR + h) * TILE + ls]; }
     });
 }
-// bring x, z, y of the re-tiled QPs back to their home columns
+// bring x, z, y of the re-tiled QPs back to their home columns, and the t slots with them: they hold r^ of an unsolved
+// QP (mpc_common.h), which a later compaction copies from the home workspace
 template <typename T>
 static int untile_impl(mpcb_solver* s, int n, const int* list, rt_stream st) {
     const size_t S1 = (size_t)(s->prob.horizon + 1), REC = (size_t)s->REC, HDR = (size_t)s->HDR, CS = (size_t)s->CS,
                  VS = (size_t)s->VS;
-    const size_t R_X = VS + CS + (size_t)s->LT, nxp = VS + CS, NX = (size_t)s->prob.nx;
+    const size_t R_T = VS + CS + (size_t)s->LT, nxp = (size_t)s->NW + CS + VS, NX = (size_t)s->prob.nx;     // t | p | x
     T* rec = (T*)s->rec; T* hdr = (T*)s->hdr; T* yr = (T*)s->yrows;
     const T* rec2 = (const T*)s->rec2; const T* hdr2 = (const T*)s->hdr2; const T* yr2 = (const T*)s->yrows2;
     const int per = (int)(S1 * (nxp + CS) + 2 * NX);
@@ -446,8 +447,8 @@ static int untile_impl(mpcb_solver* s, int n, const int* list, rt_stream st) {
         const int b = list[j];
         const size_t td = (size_t)(b >> 5), ldn = (size_t)(b & 31), ts = (size_t)(j >> 5), ls = (size_t)(j & 31);
         size_t r = (size_t)e;
-        if (r < S1 * nxp) {                      // x and p (= z) blocks of every record
-            const size_t k = r / nxp, o = R_X + (r - k * nxp);
+        if (r < S1 * nxp) {                      // t, p (= z) and x blocks of every record
+            const size_t k = r / nxp, o = R_T + (r - k * nxp);
             rec[((td * S1 + k) * REC + o) * TILE + ldn] = rec2[((ts * S1 + k) * REC + o) * TILE + ls];
             return;
         }
