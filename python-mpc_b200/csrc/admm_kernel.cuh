@@ -8,9 +8,11 @@
 //                     the whole record of the next stage, completion tracked by an mbarrier per buffer; all writes go
 //                     straight to global memory.  Persistent CTAs; the warps of a CTA take (chunk, tile) work items
 //                     together and meet at a CTA barrier once per iteration (instruction-cache sharing).
-//   Both drive the same stage functions (qp_thread.cuh): forward / backward sweep (first-iteration and save-old
-//   variants as template instantiations) and ONE termination-sweep body that serves the residuals and, on a second
-//   pass over (dx, dy), the infeasibility certificates.
+//   Both drive the same stage functions (qp_thread.cuh): forward / backward sweep, with first-iteration and tested-iteration
+//   variants as template instantiations.  The backward sweep of a tested iteration (kBwdTest) also evaluates the
+//   termination test — the residuals of (x, y) and the infeasibility certificates of (dx, dy) — from what it holds anyway:
+//   the new state in registers, the old one in the record it reads.  A tested iteration therefore costs no memory traffic
+//   beyond its two sweeps, and needs no copy of the old state.
 #pragma once
 #include "qp_thread.cuh"
 #include <type_traits>
@@ -40,40 +42,6 @@ MPCB_HD void admm_cold_start(const KParams<T>& p, const Ws<T, L>& ws) {
     for (int i = 0; i < L::NX; ++i) { MPCB_AT(ws.hdr, L::H_P0 + i) = 0; MPCB_AT(ws.hdr, L::H_Y0 + i) = 0; }
 }
 
-// An iteration that ends with a termination test first copies x and the row state of every stage (and the dyn_0
-// rows of the header) into the old-state buffer: the infeasibility certificates need delta-x / delta-y of exactly
-// this iteration.  A global->global copy outside the sweeps (their code and register allocation stay untouched), a
-// stage's 22 loads in flight together; 1 iteration in `check_termination` pays 2 x 22 elements per stage (~1 % of
-// the traffic).  Out of line on the GPU: scalar arguments only, so the call costs nothing worth mentioning.
-template <typename T, typename L>
-#if defined(__CUDACC__) && !defined(MPCB_EMU)
-__device__ __noinline__
-#else
-inline
-#endif
-void admm_save_old_raw(const T* rec, T* scr, const T* hdr, T* scr_hdr, int N) {
-    constexpr int NE = L::VS + L::CS;
-    for (int k = 0; k <= N; ++k) {
-        const T* R = rec + (size_t)k * L::REC * TILE;
-        T* O = scr + (size_t)k * NE * TILE;
-        T tmp[NE];       // [x | p], the order of the old-state buffer
-#pragma unroll
-        for (int e = 0; e < L::VS; ++e) tmp[e] = MPCB_AT(R, L::R_X + e);
-#pragma unroll
-        for (int e = 0; e < L::CS; ++e) tmp[L::VS + e] = MPCB_AT(R, L::R_P + e);
-#pragma unroll
-        for (int e = 0; e < NE; ++e) MPCB_AT(O, e) = tmp[e];
-    }
-    T t0[L::NX];
-#pragma unroll
-    for (int i = 0; i < L::NX; ++i) t0[i] = MPCB_AT(hdr, L::H_P0 + i);
-#pragma unroll
-    for (int i = 0; i < L::NX; ++i) MPCB_AT(scr_hdr, i) = t0[i];
-}
-template <typename T, typename L>
-MPCB_HD void admm_save_old_all(const KParams<T>& p, const Ws<T, L>& ws) {
-    admm_save_old_raw<T, L>(ws.rec, ws.scr, ws.hdr, ws.scr_hdr, p.N);
-}
 template <typename T>
 MPCB_HD bool admm_is_tested(const KParams<T>& p, int it) {
     return (p.check_every > 0 && (it % p.check_every == 0)) || it == p.max_iter;
@@ -92,7 +60,7 @@ MPCB_HD void admm_fwd_begin(const KParams<T>& p, const AdmmConst<T, L>& q, int b
     }
 }
 
-// start of a termination sweep: rows dyn_0 (header)
+// start of a termination sweep of the CTA and dense kernels: rows dyn_0 (header)
 template <typename T, typename L>
 MPCB_HD void admm_test_begin(const KParams<T>& p, const AdmmConst<T, L>& q, int b, const T* H, TestCarry<T, L>& cy,
                              TestAcc<T>& t, bool cert, bool first, const T* O0) {
@@ -119,7 +87,7 @@ MPCB_HD void test_to_cert(const TestAcc<T>& t, Cert<T>& c) {
 
 // osqp.c / auxil.c: the decision taken after a residual evaluation, in two steps.
 //   admm_residual_test: true when the exact residual test passes (status solved — OSQP evaluates no certificate
-//   then); otherwise the certificate sweep is run and admm_decide concludes.
+//   then); otherwise the certificates are consulted and admm_decide concludes.
 template <typename T, typename L>
 MPCB_HD bool admm_residual_test(const KParams<T>& p, const AdmmConst<T, L>& q, Resid<T>& rs) {
     rs.dua *= q.cinv;
@@ -141,7 +109,7 @@ MPCB_HD int admm_test(const KParams<T>& p, const AdmmConst<T, L>& q, const Resid
     if (prim_ok && dual_ok) return approx ? kSolvedInaccurate : kSolved;
     return 0;
 }
-// after the certificate sweep of a QP that failed the residual test (rs.dua already unscaled by admm_residual_test).
+// after the certificates of a QP that failed the residual test (rs.dua already unscaled by admm_residual_test).
 // Returns true when the loop ends.
 template <typename T, typename L>
 MPCB_HD bool admm_decide(const KParams<T>& p, const AdmmConst<T, L>& q, const Resid<T>& rs, const Cert<T>& ct, bool at_cap,
@@ -193,9 +161,8 @@ MPCB_HD void admm_finish(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T,
 }
 
 // Forward and backward sweep of one iteration straight out of global memory.  FIRST (iteration 1 of a solve: rows
-// enter as explicit (z, y)), RHS (the forward sweep starts from r^) and SAVE (the next iteration is tested: duplicate the
-// new state into the old-state buffer) are template parameters: the steady-state instantiation carries none of that code
-// or state.
+// enter as explicit (z, y)), RHS (the forward sweep starts from r^) and MODE (kBwdTest: the iteration is tested) are
+// template parameters: the steady-state instantiation carries none of that code or state.
 template <typename T, typename L, bool FIRST, bool RHS = false>
 MPCB_HD void admm_one_fwd(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T, L>& m, int bi, const Ws<T, L>& ws) {
     FwdCarry<T, L> cy;
@@ -205,19 +172,34 @@ MPCB_HD void admm_one_fwd(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T
         admm_fwd_stage<T, L, FIRST, RHS>(p, q, m, bi, k, ws.R(k), ws.Y(k), ws.R(k), cy);
     }
 }
-template <typename T, typename L, bool FIRST, bool SAVE>
-MPCB_HD void admm_one_bwd(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T, L>& m, int bi, const Ws<T, L>& ws) {
+template <typename T, typename L, bool FIRST, int MODE>
+MPCB_HD void admm_one_bwd(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T, L>& m, int bi, const Ws<T, L>& ws,
+                          BwdTest<T, L>& ts) {
     BwdCarry<T, L> cy;
 #pragma unroll
     for (int i = 0; i < L::NX; ++i) { cy.xt_next[i] = 0; cy.Dx_next[i] = 1; }
+    if (MODE == kBwdTest) test_reset(ts);
     for (int k = p.N; k >= 0; --k) {
         if (p.tv && k < p.N) load_model<T, L>(p, bi, k, m);
-        admm_bwd_stage<T, L, FIRST, SAVE>(p, q, m, bi, k, ws.R(k), ws.Y(k), ws.R(k), cy, ws.S(k));
+        admm_bwd_stage<T, L, FIRST, MODE>(p, q, m, bi, k, ws.R(k), ws.Y(k), ws.R(k), cy, ts);
     }
-    admm_bwd_header<T, L, FIRST, SAVE>(p, q, bi, ws.hdr, cy, ws.scr_hdr);
+    admm_bwd_header<T, L, FIRST, MODE>(p, q, bi, ws.hdr, cy, ts);
 }
-// Where the old state of a tested iteration `it` comes from: the backward sweep of iteration it-1 (SAVE) when that was a
-// steady-state iteration, else (it <= 2: the state a solve starts from, or the one its first iteration left) a copy.
+// The termination test of a tested iteration, after its backward sweep (kBwdTest) accumulated ts.  Returns true when the
+// QP's loop ends (status set).  The certificates are consulted only when the residual test fails, as in OSQP.
+template <typename T, typename L>
+MPCB_HD bool admm_conclude(const KParams<T>& p, const AdmmConst<T, L>& q, const BwdTest<T, L>& ts, int it, Resid<T>& rs,
+                           int& status) {
+    test_to_resid(ts.r, rs);
+    if (admm_residual_test<T, L>(p, q, rs)) { status = kSolved; return true; }
+    if (!p.certs && it != p.max_iter) return false;
+    Cert<T> ct;
+    test_to_cert(ts.c, ct);
+    return admm_decide<T, L>(p, q, rs, ct, it == p.max_iter, status);
+}
+// The CTA and dense kernels evaluate the certificates of a tested iteration `it` in a sweep of their own, from a copy of
+// the old state: made by the backward sweep of iteration it-1 when that was a steady-state iteration, else (it <= 2: the
+// state a solve starts from, or the one its first iteration left) before the iteration.
 template <typename T>
 MPCB_HD bool admm_saves(const KParams<T>& p, int it) { return it >= 2 && admm_is_tested(p, it + 1); }
 template <typename T>
@@ -225,7 +207,6 @@ MPCB_HD bool admm_needs_copy(const KParams<T>& p, int it) { return it <= 2 && ad
 
 template <typename T, typename L>
 MPCB_HD void admm_one(const KParams<T>& p, int b) {
-    const int N = p.N;
     const int bi = p.qp_map ? p.qp_map[b] : b;          // QP index for inputs and outputs; b is the workspace slot
     if (p.status[bi] != kUnsolved) return;               // solved in an earlier chunk, or not factorable (-7)
     Ws<T, L> ws(p, b);
@@ -237,48 +218,24 @@ MPCB_HD void admm_one(const KParams<T>& p, int b) {
     int status = kUnsolved, it = 0;
     Resid<T> rs;
     rs.pri = rs.dua = 0;
+    BwdTest<T, L> ts;
     for (it = p.it0 + 1; it <= p.it_stop; ++it) {
-        const bool first = (it == 1);
-        if (admm_needs_copy(p, it)) admm_save_old_all<T, L>(p, ws);
-        if (first) { admm_one_fwd<T, L, true>(p, q, m, bi, ws); admm_one_bwd<T, L, true, false>(p, q, m, bi, ws); }
-        else {
+        const bool tested = admm_is_tested(p, it);
+        if (it == 1) {
+            admm_one_fwd<T, L, true>(p, q, m, bi, ws);
+            if (tested) admm_one_bwd<T, L, true, kBwdTest>(p, q, m, bi, ws, ts);
+            else admm_one_bwd<T, L, true, kBwdPlain>(p, q, m, bi, ws, ts);
+        } else {
             if (p.fwd_rhs) admm_one_fwd<T, L, false, true>(p, q, m, bi, ws);
             else admm_one_fwd<T, L, false>(p, q, m, bi, ws);
-            if (admm_saves(p, it)) admm_one_bwd<T, L, false, true>(p, q, m, bi, ws);
-            else admm_one_bwd<T, L, false, false>(p, q, m, bi, ws);
+            if (tested) admm_one_bwd<T, L, false, kBwdTest>(p, q, m, bi, ws, ts);
+            else admm_one_bwd<T, L, false, kBwdPlain>(p, q, m, bi, ws, ts);
         }
-        if (admm_is_tested(p, it)) {
-            bool done = false;
-            for (int pass = 0; pass < 2 && !done; ++pass) {     // residuals of (x, y), then certificates of (dx, dy)
-                const bool cert = pass == 1;
-                TestCarry<T, L> cy;
-                TestAcc<T> t;
-                admm_test_begin<T, L>(p, q, bi, ws.hdr, cy, t, cert, first, ws.scr_hdr);
-                for (int k = 0; k <= N; ++k) {
-                    if (p.tv && k < N) load_model<T, L>(p, bi, k, m);
-                    admm_test_stage<T, L>(p, q, m, bi, k, ws.R(k), ws.R(k < N ? k + 1 : k), cy, t, cert, first, ws.Y(k),
-                                          ws.S(k), ws.S(k < N ? k + 1 : k));
-                }
-                if (!cert) {
-                    test_to_resid(t, rs);
-                    if (admm_residual_test<T, L>(p, q, rs)) { status = kSolved; done = true; }
-                    else if (!p.certs && it != p.max_iter) break;
-                } else {
-                    Cert<T> ct;
-                    test_to_cert(t, ct);
-                    if (admm_decide<T, L>(p, q, rs, ct, it == p.max_iter, status)) done = true;
-                }
-            }
-            if (done) break;
-        }
+        if (tested && admm_conclude<T, L>(p, q, ts, it, rs, status)) break;
     }
     admm_finish<T, L>(p, q, m, ws, bi, status, it > p.it_stop ? p.it_stop : it, rs);
 }
 
-
-#ifndef MPCB_SAVE_BY_COPY
-#define MPCB_SAVE_BY_COPY 0      // measured (r2): 26.0 ms per step with the copy, 25.8 ms with the SAVE instantiation — kept off
-#endif
 #if defined(__CUDACC__) && !defined(MPCB_EMU)
 // ==============================================================================================
 // Warp-per-tile ADMM with the stage records staged through shared memory by TMA bulk copies.
@@ -312,7 +269,7 @@ __device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.
 
 // What a TMA load of a stage record brings into a record buffer (one mbarrier transaction, one or two bulk copies):
 //   kLoadAll  the whole record: the backward sweep, and stage 0 / stage N of a forward sweep (the backward turn-around)
-//   kLoadFwd  all but t: a forward sweep that forms the whole right-hand side, and the termination sweep
+//   kLoadFwd  all but t: a forward sweep that forms the whole right-hand side
 //   kLoadRhs  the runs FA and FB: a forward sweep that starts from r^ (mpc_common.h)
 enum { kLoadAll, kLoadFwd, kLoadRhs };
 template <typename T, typename L, int WHAT>
@@ -335,7 +292,7 @@ __device__ __forceinline__ void tma_load_stage(T* dst, const T* src, unsigned lo
 // Forward and backward sweep of one iteration of a tile: record k is resident in one of the warp's two buffers while
 // the elected lane has the TMA bulk load of the next record in flight into the other.  FIRST = iteration 1 of a solve
 // (rows enter as explicit (z, y)), RHS = the forward sweep starts from r^ and loads only the runs FA and FB of the
-// records in between, SAVE = the next iteration is tested (the new state is duplicated into the old-state buffer); the
+// records in between, MODE = kBwdTest: the iteration is tested (the backward sweep accumulates the test into ts); the
 // steady-state instantiation carries none of that code or state.  Record 0 of a forward sweep is resident whole (the
 // backward turn-around patches it, or a kLoadAll), so is record N (loaded whole for the backward turn-around).
 template <typename T, typename L, bool FIRST, bool RHS>
@@ -371,10 +328,11 @@ __device__ __forceinline__ void admm_tma_fwd(const KParams<T>& p, const AdmmCons
     }
 #undef MPCB_BUF
 }
-template <typename T, typename L, bool FIRST, bool SAVE>
+template <typename T, typename L, bool FIRST, int MODE>
 __device__ __forceinline__ void admm_tma_bwd(const KParams<T>& p, const AdmmConst<T, L>& q, Model<T, L>& m,
                                              const Ws<T, L>& ws, int bb, int lane, bool active, T* buf0,
-                                             unsigned long long* bar, unsigned& ph, int& cur, const T* rec_tile) {
+                                             unsigned long long* bar, unsigned& ph, int& cur, const T* rec_tile,
+                                             BwdTest<T, L>& ts) {
     const int N = p.N;
 #define MPCB_BUF(c) (buf0 + (c) * (L::REC * TILE))
     // ---------------- backward sweep: record N is resident in MPCB_BUF(cur); prefetch k-1 (with t)
@@ -382,13 +340,14 @@ __device__ __forceinline__ void admm_tma_bwd(const KParams<T>& p, const AdmmCons
         BwdCarry<T, L> cy;
 #pragma unroll
         for (int i = 0; i < L::NX; ++i) { cy.xt_next[i] = 0; cy.Dx_next[i] = 1; }
+        if (MODE == kBwdTest) test_reset(ts);
         for (int k = N; k >= 0; --k) {
             if (k > 0 && lane == 0)
                 tma_load_stage<T, L, kLoadAll>(MPCB_BUF(cur ^ 1), rec_tile + (size_t)(k - 1) * L::REC * TILE, &bar[cur ^ 1]);
             if (k < N) { mbar_wait(&bar[cur], (ph >> cur) & 1u); ph ^= 1u << cur; }
             if (active) {
                 if (p.tv && k < N) load_model<T, L>(p, bb, k, m);
-                admm_bwd_stage<T, L, FIRST, SAVE>(p, q, m, bb, k, MPCB_BUF(cur) + lane, ws.Y(k), ws.R(k), cy, ws.S(k));
+                admm_bwd_stage<T, L, FIRST, MODE>(p, q, m, bb, k, MPCB_BUF(cur) + lane, ws.Y(k), ws.R(k), cy, ts);
                 if (k == 0) {                     // turn-around: the next forward stage 0 reuses this buffer: new r^, p, x
 #pragma unroll
                     for (int e = 0; e < L::NW + L::CS + L::VS; ++e)
@@ -399,7 +358,7 @@ __device__ __forceinline__ void admm_tma_bwd(const KParams<T>& p, const AdmmCons
             __syncwarp();
             if (k > 0) cur ^= 1;
         }
-        if (active) admm_bwd_header<T, L, FIRST, SAVE>(p, q, bb, ws.hdr, cy, ws.scr_hdr);
+        if (active) admm_bwd_header<T, L, FIRST, MODE>(p, q, bb, ws.hdr, cy, ts);
     }
 #undef MPCB_BUF
 }
@@ -409,7 +368,7 @@ __global__ void __launch_bounds__(256, 1) admm_tma_kernel(const __grid_constant_
     extern __shared__ __align__(128) unsigned char smem_raw[];
     constexpr unsigned REC_BYTES = L::REC * TILE * sizeof(T);
     const int warps = blockDim.x >> 5, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int N = p.N, ntiles = (p.B + TILE - 1) / TILE;
+    const int ntiles = (p.B + TILE - 1) / TILE;
     T* const buf0 = reinterpret_cast<T*>(smem_raw + (size_t)warp * 2 * REC_BYTES);     // two record buffers of this warp
 #define MPCB_BUF(c) (buf0 + (c) * (L::REC * TILE))
     unsigned long long* bar = reinterpret_cast<unsigned long long*>(smem_raw + (size_t)warps * 2 * REC_BYTES) + warp * 2;
@@ -429,10 +388,11 @@ __global__ void __launch_bounds__(256, 1) admm_tma_kernel(const __grid_constant_
     // dependency — chunk c of a tile after its chunk c-1 — is tracked in tile_prog[] (release/acquire).
     //
     // The warps of a CTA take their items TOGETHER (one round = `warps` consecutive items) and meet at a CTA barrier
-    // once per iteration.  The sweeps are ~35 KB of straight-line code and the termination sweep another ~50 KB that
-    // a warp walks once per 25 iterations: with the warps in step each fetched instruction line serves all of them,
-    // out of step the rarely run code is an instruction-cache miss from end to end (measured: `no_instruction` was
-    // 70 % of the termination sweep's stall samples and a third of the sweeps').  Every barrier below is reached by
+    // once per iteration.  The sweeps are long straight-line code, and the tested backward sweep is a variant that a warp
+    // walks once per check_termination iterations: with the warps in step each fetched instruction line serves all of
+    // them, out of step the rarely run code is an instruction-cache miss from end to end (measured, round 1:
+    // `no_instruction` was 70 % of the then separate termination sweep's stall samples and a third of the sweeps').
+    // Every barrier below is reached by
     // every thread of the CTA the same number of times: base, total_items and chunk_len are CTA-uniform, and a warp
     // without work (no item, nothing left in its tile, all its QPs done) keeps walking the round's barriers.
     const int span = p.it_stop - p.it0;
@@ -496,86 +456,29 @@ __global__ void __launch_bounds__(256, 1) admm_tma_kernel(const __grid_constant_
             mbar_wait(&bar[cur], (ph >> cur) & 1u); ph ^= 1u << cur;
         }
 
+        BwdTest<T, L> ts;
         for (int r = 0; r < chunk_len; ++r) {
             const int it = it_begin + 1 + r;
             const bool run = alive && it <= it_end;
             if (!__syncthreads_or(run)) break;           // CTA-uniform: nobody has an iteration left in this round
-            const bool first = (it == 1);
             if (run) {
-#if MPCB_SAVE_BY_COPY
-                // the certificates of a tested iteration need the state it starts from: copied (global -> global, 44 elements per
-                // stage once every check_termination iterations, ~1 % of the traffic) instead of duplicating the stores of the
-                // previous iteration's backward sweep — that instantiation spilled (153 M local-store sectors per solve, ncu
-                // r1n) and its code was one more ~18 KB region competing for the instruction cache
-                if (active && admm_is_tested(p, it)) admm_save_old_all<T, L>(p, ws);
-#else
-                if (active && admm_needs_copy(p, it)) admm_save_old_all<T, L>(p, ws);
-#endif
-                // ---------------- forward and backward sweep (the steady-state instantiation has no first-iteration code)
-                if (first) {
+                // ---------------- forward and backward sweep (the steady-state instantiation has no first-iteration code).
+                // A tested iteration's backward sweep evaluates the termination test; record 0 stays resident, patched by
+                // the backward turn-around, for the next forward sweep.
+                const bool tested = admm_is_tested(p, it);
+                if (it == 1) {
                     admm_tma_fwd<T, L, true, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
-                    admm_tma_bwd<T, L, true, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
+                    if (tested) admm_tma_bwd<T, L, true, kBwdTest>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile, ts);
+                    else admm_tma_bwd<T, L, true, kBwdPlain>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile, ts);
                 } else {
                     if (p.fwd_rhs) admm_tma_fwd<T, L, false, true>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
                     else admm_tma_fwd<T, L, false, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
-#if MPCB_SAVE_BY_COPY
-                    admm_tma_bwd<T, L, false, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
-#else
-                    if (admm_saves(p, it)) admm_tma_bwd<T, L, false, true>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
-                    else admm_tma_bwd<T, L, false, false>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile);
-#endif
+                    if (tested) admm_tma_bwd<T, L, false, kBwdTest>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile, ts);
+                    else admm_tma_bwd<T, L, false, kBwdPlain>(p, q, m, ws, bb, lane, active, buf0, bar, ph, cur, rec_tile, ts);
                 }
-            }
-            // ---------------- termination test, staged like the sweeps.  Stage k needs records k and k+1 (x_{k+1}
-            // enters row dyn_{k+1}), so both buffers are resident while it is evaluated and the TMA latency of each
-            // load is exposed — once every check_termination iterations.  Pass 0: the residuals; pass 1 (only if a QP
-            // of the tile failed the residual test): the infeasibility certificates, the same code over (dx, dy).
-            const bool my_test = run && admm_is_tested(p, it);
-            if (!__syncthreads_or(my_test)) continue;    // CTA-uniform; the warps enter the termination sweep together
-            if (my_test) {
-                bool open_ = active;                          // lanes the current pass evaluates
-                for (int pass = 0; pass < 2; ++pass) {
-                    const bool cert = pass == 1;
-                    TestCarry<T, L> cy;
-                    TestAcc<T> t;
-                    if (open_) admm_test_begin<T, L>(p, q, bb, ws.hdr, cy, t, cert, first, ws.scr_hdr);   // buffer `cur` holds record 0
-                    for (int k = 0; k <= N; ++k) {
-                        if (k < N) {
-                            if (lane == 0)
-                                tma_load_stage<T, L, kLoadFwd>(MPCB_BUF(cur ^ 1), rec_tile + (size_t)(k + 1) * L::REC * TILE, &bar[cur ^ 1]);
-                            mbar_wait(&bar[cur ^ 1], (ph >> (cur ^ 1)) & 1u); ph ^= 1u << (cur ^ 1);
-                        }
-                        if (open_) {
-                            if (p.tv && k < N) load_model<T, L>(p, bb, k, m);
-                            admm_test_stage<T, L>(p, q, m, bb, k, MPCB_BUF(cur) + lane, MPCB_BUF(k < N ? cur ^ 1 : cur) + lane, cy, t,
-                                                  cert, first, ws.Y(k), ws.S(k), ws.S(k < N ? k + 1 : k));
-                        }
-                        __syncwarp();
-                        if (k < N) cur ^= 1;
-                    }
-                    if (open_) {
-                        if (!cert) {
-                            test_to_resid(t, rs);
-                            if (admm_residual_test<T, L>(p, q, rs)) { status = kSolved; active = false; it_done = it; open_ = false; }
-                            else if (!p.certs && it != p.max_iter) open_ = false;
-                        } else {
-                            Cert<T> ct;
-                            test_to_cert(t, ct);
-                            if (admm_decide<T, L>(p, q, rs, ct, it == p.max_iter, status)) { active = false; it_done = it; }
-                        }
-                    }
-                    if (cert || !__any_sync(0xffffffffu, open_)) break;
-                    // the certificate pass starts again from record 0
-                    if (lane == 0) tma_load_stage<T, L, kLoadFwd>(MPCB_BUF(cur ^ 1), rec_tile, &bar[cur ^ 1]);
-                    mbar_wait(&bar[cur ^ 1], (ph >> (cur ^ 1)) & 1u); ph ^= 1u << (cur ^ 1);
-                    cur ^= 1;
-                }
-                if (!__any_sync(0xffffffffu, active)) alive = false;     // every QP of the tile is done: no more sweeps
-                else {
-                    // the next forward sweep expects record 0 (whole, r^ included) in the current buffer
-                    if (lane == 0) tma_load_stage<T, L, kLoadAll>(MPCB_BUF(cur ^ 1), rec_tile, &bar[cur ^ 1]);
-                    mbar_wait(&bar[cur ^ 1], (ph >> (cur ^ 1)) & 1u); ph ^= 1u << (cur ^ 1);
-                    cur ^= 1;
+                if (tested) {
+                    if (active && admm_conclude<T, L>(p, q, ts, it, rs, status)) { active = false; it_done = it; }
+                    if (!__any_sync(0xffffffffu, active)) alive = false;     // every QP of the tile is done: no more sweeps
                 }
             }
         }

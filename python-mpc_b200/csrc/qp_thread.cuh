@@ -8,7 +8,7 @@
 //               slack variables are eliminated in closed form) as a block-bidiagonal Cholesky;
 //               stores the inverse diagonal blocks Linv_k only: the coupling blocks
 //               F_k = C_k Linv_k' are re-applied from the model and the scalings    -> Linv
-//   admm_fwd_stage / admm_bwd_stage / admm_check_stage / admm_exit_stage
+//   admm_fwd_stage / admm_bwd_stage / admm_test_stage / admm_exit_stage
 //               one stage of the OSQP ADMM loop (osqp.c: update_xz_tilde / update_x / update_z /
 //               update_y; auxil.c: check_termination) with fixed rho / sigma / alpha.  The loop that
 //               drives them (and stages the records through shared memory with TMA bulk copies on
@@ -693,15 +693,93 @@ struct BwdCarry {
     T Dx_next[L::NX];    // D_x(k+1)
 };
 
-// SAVE: the next iteration ends with a termination test — the new x and row state also go to the old-state buffer O
-// (what the infeasibility certificates of that iteration call x^{k-1}, y^{k-1}); duplicate stores, nothing else.
+// ---- termination test on the unscaled residuals (auxil.c: check_termination), one stage
+template <typename T>
+struct Resid {
+    T pri, dua, nz, nAx, nq, nAty, nPx;
+};
+// The accumulators of one evaluation of the termination test.  ONE set of terms serves both evaluations OSQP makes at a
+// termination test:
+//   the residuals of (x, y)                                        (auxil.c: compute_pri_res / compute_dua_res, tolerances)
+//   the infeasibility certificates of (dx, dy) = (x - x_old, y - y_old)   (is_primal/dual_infeasible)
+// Both need the same linear forms — E^-1 A v by rows, D^-1 A'w and D^-1 P v by columns — applied to v = x, w = y or to
+// v = dx, w = dy.
+template <typename T>
+struct TestAcc {
+    T pri, dua, nz, nAx, nq, nAty, nPx;      // residual norms; nAty = ||D^-1 A'w||, nPx = ||D^-1 P v|| serve both evaluations
+    T nEw, lhs, nDv, qv, aup, alo;           // certificate terms: ||E w||, u'w+ + l'w-, ||D v||, q'v, max / min of E^-1 A v
+};
+template <typename T>
+MPCB_HD void test_reset(TestAcc<T>& a) {
+    a.pri = a.dua = a.nz = a.nAx = a.nq = a.nAty = a.nPx = 0;
+    a.nEw = a.lhs = a.nDv = a.qv = 0;
+    a.aup = (T)-kOsqpInfty; a.alo = (T)kOsqpInfty;
+}
+// is_primal_infeasible projects dy on the recession cone of the row's bound type first
+template <typename T>
+MPCB_HD T cert_project(bool inf_possible, T dy, T lb, T ub) {
+    if (inf_possible) {
+        const bool up_inf = ub > (T)(kOsqpInfty * kMinScaling), lo_inf = lb < (T)(-kOsqpInfty * kMinScaling);
+        if (up_inf && lo_inf) dy = 0;
+        else if (up_inf) dy = tmin(dy, (T)0);
+        else if (lo_inf) dy = tmax(dy, (T)0);
+    }
+    return dy;
+}
+
+// The termination test of a tested iteration, evaluated by its backward sweep (admm_bwd_stage in mode kBwdTest).  At stage k
+// the sweep holds the new x_k and p in registers and the old ones — x^{k-1}, y^{k-1} of the certificates — in the record it
+// reads.  Every norm is a max-norm except lhs and qv, so the order of the stages does not matter.  A stage's row dyn_{k+1}
+// needs the new x_{k+1}, and the dual residual of column x_k needs the new row dyn_k, which stage k-1 forms: both are
+// carried here.  `r` gets the residual terms of (x, y), `c` the certificate terms of (dx, dy); admm_test_stage evaluates the
+// same expressions.
+template <typename T, typename L>
+struct BwdTest {
+    TestAcc<T> r, c;
+    T x_next[L::NX], dx_next[L::NX];              // new x_{k+1}, x_{k+1} - x_{k+1}^old
+    T own_r[L::NX], qpx_r[L::NX], own_c[L::NX];   // column x_{k+1} without its row dyn_{k+1}: A'y part, q + P x; A'dy part
+};
+enum { kBwdPlain, kBwdTest };
+// A copy of v that the compiler cannot trace back to v's expression.  The test terms form their products from such copies
+// so that they share none with the iterate arithmetic: the compiler fuses a product into an FMA only when every use of it
+// is an addition, so one more use by the test would change how the tested iteration's iterates round.
+MPCB_HD float opaque(float v) {
+#ifdef __CUDA_ARCH__
+    asm("" : "+f"(v));
+#endif
+    return v;
+}
+MPCB_HD double opaque(double v) {
+#ifdef __CUDA_ARCH__
+    asm("" : "+d"(v));
+#endif
+    return v;
+}
+template <typename T, typename L>
+MPCB_HD void test_reset(BwdTest<T, L>& ts) { test_reset(ts.r); test_reset(ts.c); }
+// the dual residual of column x_{k+1} (carried) once its row dyn_{k+1} is known: E y of that row is wr times the row's E,
+// ex = E_dyn(k+1) D_x(k+1)
+template <typename T, typename L>
+MPCB_HD void test_close_column(BwdTest<T, L>& ts, int i, T ex, T wr, T wc, T Dinv) {
+    T atyr = ts.own_r[i], atyc = ts.own_c[i];
+    atyr -= ex * wr;
+    atyc -= ex * wc;
+    ts.r.dua = tmax(ts.r.dua, tabs(Dinv * (ts.qpx_r[i] + atyr)));
+    ts.r.nAty = tmax(ts.r.nAty, tabs(Dinv * atyr));
+    ts.c.nAty = tmax(ts.c.nAty, tabs(Dinv * atyc));
+}
+
+// MODE kBwdTest: the iteration ends with a termination test, accumulated into ts (BwdTest); the iterate arithmetic and the
+// stores are those of kBwdPlain.
 // Every instantiation leaves r^_k in the t slots of R: the part of the next forward sweep's right-hand side r_k that depends
 // on stage k alone (sigma x, the cost term, the bound rows and the slack elimination, A'w / B'w of rows dyn_{k+1}), formed
 // from the new x_k and the new p-form rows — all in registers here, while the next forward sweep would have to read them.
-template <typename T, typename L, bool FIRST, bool SAVE>
+// S may alias R (the lane-per-QP kernel): every old value is read before the stage writes it.
+template <typename T, typename L, bool FIRST, int MODE>
 MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const Model<T, L>& m, int b, int k,
-                            const T* S, const T* Yk, T* R, BwdCarry<T, L>& cy, T* O) {
+                            const T* S, const T* Yk, T* R, BwdCarry<T, L>& cy, BwdTest<T, L>& ts) {
     constexpr bool first = FIRST;
+    constexpr bool TEST = MODE == kBwdTest;
     constexpr int NX = L::NX, NU = L::NU, NW = L::NW, NS = L::NS;
     const bool last = (k == p.N);
     T lo[NX], hi[NX];
@@ -747,32 +825,36 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
     }
     // rows bx_k (+ slack recovery), x_k / s_k
     T rh[NW];         // r^_k
+    // kBwdTest: the new x_k, u_k and their deltas; the columns x_k / u_k until the new rows dyn_{k+1} are known
+    T xn_a[NX], dx_a[NX], ownr_x[NX], ownc_x[NX], qpx_x[NX], un_a[NU], du_a[NU], ownr_u[NU], ownc_u[NU], pxr_u[NU];
+    (void)xn_a; (void)dx_a; (void)ownr_x; (void)ownc_x; (void)qpx_x; (void)un_a; (void)du_a; (void)ownr_u; (void)ownc_u;
+    (void)pxr_u;
 #pragma unroll
     for (int j = 0; j < NX; ++j) {
         const T Ebx = MPCB_AT(S, L::R_E + L::OBX + j);
         const T bx = Ebx * Dx[j], lb = Ebx * lo[j], ub = Ebx * hi[j];
         const T rb = row_rho(q.inf_bounds, lb, ub, q.rho, q.rho_eq);
         const Row<T> rw = row_state_b(first, MPCB_AT(S, L::R_P + L::OBX + j), Yk + (L::OBX + j) * TILE, lb, ub, rb, q);
+        const T xo = TEST ? MPCB_AT(S, L::R_X + L::OX + j) : (T)0;     // (old x_k; S may alias R)
         T ztil = bx * w[j];
-        T sn = 0, bs = 0, mxs = 0, mss = 1;
+        T sn = 0, bs = 0, mxs = 0, mss = 1, so = 0;
         if (NS) {
             const T Dsl = MPCB_AT(S, L::R_D + L::OS + (NS ? j : 0));
             bs = p.S[j] * Ebx * Dsl;
             mss = q.c * p.W[j] * Dsl * Dsl + q.sigma + rb * bs * bs;
             mxs = rb * bx * bs;
             const T sold = MPCB_AT(S, L::R_X + L::OS + (NS ? j : 0));
+            if (TEST) so = sold;
             const T rs = q.sigma * sold + bs * (rb * (rw.z - rw.yr));
             const T st = (rs - mxs * w[j]) * fast_rcp(mss);
             ztil += bs * st;
             sn = q.alpha * st + ((T)1 - q.alpha) * sold;
             MPCB_AT(R, L::R_X + L::OS + (NS ? j : 0)) = sn;
-            if (SAVE) MPCB_AT(O, L::OS + (NS ? j : 0)) = sn;
         }
         const T pn = row_next(ztil, rw, q.alpha);
         const T xn = q.alpha * w[j] + ((T)1 - q.alpha) * MPCB_AT(S, L::R_X + L::OX + j);
         MPCB_AT(R, L::R_P + L::OBX + j) = pn;
         MPCB_AT(R, L::R_X + L::OX + j) = xn;
-        if (SAVE) { MPCB_AT(O, L::VS + L::OBX + j) = pn; MPCB_AT(O, L::OX + j) = xn; }
         // r^: sigma x - q + bx' (rho (z - y/rho)) of the new state, minus the slack elimination (A'w of rows dyn_{k+1} below)
         const Row<T> rn = row_state(false, pn, (T)0, lb, ub, (T)0);
         const T vbx = rb * (rn.z - rn.yr);
@@ -781,9 +863,47 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
         T v = q.sigma * xn - qh + bx * vbx;
         if (NS) v -= mxs * fast_rcp(mss) * (q.sigma * sn + bs * vbx);
         rh[j] = v;
+        if (TEST) {       // row bx_k and columns s_k; column x_k without the rows dyn_k, dyn_{k+1}
+            const T Einv = fast_rcp(Ebx), Dinv = fast_rcp(Dx[j]);
+            const T vx = xn - xo, vs = sn - so;
+            T wr = rb * (pn - rn.z);
+            T wc = wr;
+            wc -= rb * rw.yr;
+            wc = cert_project(q.inf_bounds, wc, lb, ub);
+            const T axr = bx * xn + bs * sn, axc = bx * vx + bs * vs;
+            ts.r.pri = tmax(ts.r.pri, tabs(Einv * (axr - rn.z)));
+            ts.r.nz = tmax(ts.r.nz, tabs(Einv * rn.z));
+            ts.r.nAx = tmax(ts.r.nAx, tabs(Einv * axr));
+            if (!q.inf_bounds || ub < (T)(kOsqpInfty * kMinScaling)) ts.c.aup = tmax(ts.c.aup, Einv * axc);
+            if (!q.inf_bounds || lb > (T)(-kOsqpInfty * kMinScaling)) ts.c.alo = tmin(ts.c.alo, Einv * axc);
+            ts.c.nEw = tmax(ts.c.nEw, tabs(Ebx * wc));
+            ts.c.lhs += ub * tmax(wc, (T)0) + lb * tmin(wc, (T)0);
+            const T Qkj = (last ? p.QN : p.Q)[j];
+            const T qt = q.c * Dx[j] * (-(Qkj * opaque(xr)));      // = qh
+            const T pxr = q.c * Qkj * Dx[j] * Dx[j] * xn, pxc = q.c * Qkj * Dx[j] * Dx[j] * vx;
+            ts.r.nq = tmax(ts.r.nq, tabs(Dinv * qt));
+            ts.r.nPx = tmax(ts.r.nPx, tabs(Dinv * pxr));
+            ts.c.nPx = tmax(ts.c.nPx, tabs(Dinv * pxc));
+            ts.c.nDv = tmax(ts.c.nDv, tabs(Dx[j] * vx));
+            ts.c.qv += qt * vx;
+            xn_a[j] = xn; dx_a[j] = vx; ownr_x[j] = bx * wr; ownc_x[j] = bx * wc; qpx_x[j] = qt + pxr;
+            if (NS) {
+                const T Dsl = MPCB_AT(S, L::R_D + L::OS + (NS ? j : 0)), Dsinv = fast_rcp(Dsl);
+                const T pd = q.c * p.W[j] * opaque(Dsl) * Dsl;
+                const T atys = bs * wr, pxs = pd * sn, atyc = bs * wc, pxsc = pd * vs;
+                ts.r.dua = tmax(ts.r.dua, tabs(Dsinv * (atys + pxs)));
+                ts.r.nAty = tmax(ts.r.nAty, tabs(Dsinv * atys));
+                ts.r.nPx = tmax(ts.r.nPx, tabs(Dsinv * pxs));
+                ts.c.nAty = tmax(ts.c.nAty, tabs(Dsinv * atyc));
+                ts.c.nPx = tmax(ts.c.nPx, tabs(Dsinv * pxsc));
+                ts.c.nDv = tmax(ts.c.nDv, tabs(Dsl * vs));
+            }
+        }
     }
 #pragma unroll
     for (int j = 0; j < NU; ++j) rh[NX + j] = 0;
+    T wyr[NX], wyc[NX];      // kBwdTest: E y and E dy of the new rows dyn_{k+1}
+    (void)wyr; (void)wyc;
     if (!last) {
 #pragma unroll
         for (int j = 0; j < NU; ++j) {
@@ -791,13 +911,34 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
             const T bu = Ebu * Du[j], lb = Ebu * p.umin[j], ub = Ebu * p.umax[j];
             const T rb = row_rho(q.inf_bounds, lb, ub, q.rho, q.rho_eq);
             const Row<T> rw = row_state_b(first, MPCB_AT(S, L::R_P + L::OBU + j), Yk + (L::OBU + j) * TILE, lb, ub, rb, q);
+            const T uo = TEST ? MPCB_AT(S, L::R_X + L::OU + j) : (T)0;     // (old u_k)
             const T pn = row_next(bu * w[NX + j], rw, q.alpha);
             const T un = q.alpha * w[NX + j] + ((T)1 - q.alpha) * MPCB_AT(S, L::R_X + L::OU + j);
             MPCB_AT(R, L::R_P + L::OBU + j) = pn;
             MPCB_AT(R, L::R_X + L::OU + j) = un;
-            if (SAVE) { MPCB_AT(O, L::VS + L::OBU + j) = pn; MPCB_AT(O, L::OU + j) = un; }
             const Row<T> rn = row_state(false, pn, (T)0, lb, ub, (T)0);
             rh[NX + j] = q.sigma * un + bu * (rb * (rn.z - rn.yr));
+            if (TEST) {   // row bu_k; column u_k without the rows dyn_{k+1}
+                const T Einv = fast_rcp(Ebu), Dinv = fast_rcp(Du[j]);
+                const T vu = un - uo;
+                T wr = rb * (pn - rn.z);
+                T wc = wr;
+                wc -= rb * rw.yr;
+                wc = cert_project(q.inf_bounds, wc, lb, ub);
+                const T axr = bu * un, axc = bu * vu;
+                ts.r.pri = tmax(ts.r.pri, tabs(Einv * (axr - rn.z)));
+                ts.r.nz = tmax(ts.r.nz, tabs(Einv * rn.z));
+                ts.r.nAx = tmax(ts.r.nAx, tabs(Einv * axr));
+                if (!q.inf_bounds || ub < (T)(kOsqpInfty * kMinScaling)) ts.c.aup = tmax(ts.c.aup, Einv * axc);
+                if (!q.inf_bounds || lb > (T)(-kOsqpInfty * kMinScaling)) ts.c.alo = tmin(ts.c.alo, Einv * axc);
+                ts.c.nEw = tmax(ts.c.nEw, tabs(Ebu * wc));
+                ts.c.lhs += ub * tmax(wc, (T)0) + lb * tmin(wc, (T)0);
+                const T pxr = q.c * p.R[j] * Du[j] * Du[j] * un, pxc = q.c * p.R[j] * Du[j] * Du[j] * vu;
+                ts.r.nPx = tmax(ts.r.nPx, tabs(Dinv * pxr));
+                ts.c.nPx = tmax(ts.c.nPx, tabs(Dinv * pxc));
+                ts.c.nDv = tmax(ts.c.nDv, tabs(Du[j] * vu));
+                un_a[j] = un; du_a[j] = vu; ownr_u[j] = bu * wr; ownc_u[j] = bu * wc; pxr_u[j] = pxr;
+            }
         }
         // rows dyn_{k+1}:  E (A D x~_k + B D u~_k) - ex_{k+1} x~_{k+1} = -E g_k
         T wv[NX];     // E (rho z - y) of the new rows dyn_{k+1}
@@ -814,9 +955,52 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
                                         beq, beq, q.rinv_eq());
             const T pn = row_next(ztil, rw, q.alpha);
             MPCB_AT(R, L::R_P + L::ODN + i) = pn;
-            if (SAVE) MPCB_AT(O, L::VS + L::ODN + i) = pn;
             const Row<T> rn = row_state(false, pn, (T)0, beq, beq, (T)0);
             wv[i] = Ed_next[i] * (q.rho_eq * (rn.z - rn.yr));
+            if (TEST) {   // row dyn_{k+1}; column x_{k+1} gets its row dyn_{k+1}
+                T ar = 0, ac = 0;
+#pragma unroll
+                for (int j = 0; j < NX; ++j) { ar += m.A[i][j] * (Dx[j] * xn_a[j]); ac += m.A[i][j] * (Dx[j] * dx_a[j]); }
+#pragma unroll
+                for (int j = 0; j < NU; ++j) { ar += m.B[i][j] * (Du[j] * un_a[j]); ac += m.B[i][j] * (Du[j] * du_a[j]); }
+                const T axr = Ed_next[i] * ar - exn[i] * ts.x_next[i], axc = Ed_next[i] * ac - exn[i] * ts.dx_next[i];
+                const T Einv = fast_rcp(Ed_next[i]);
+                ts.r.pri = tmax(ts.r.pri, tabs(Einv * (axr - beq)));
+                ts.r.nz = tmax(ts.r.nz, tabs(Einv * beq));
+                ts.r.nAx = tmax(ts.r.nAx, tabs(Einv * axr));
+                ts.c.aup = tmax(ts.c.aup, Einv * axc);
+                ts.c.alo = tmin(ts.c.alo, Einv * axc);
+                T wr = q.rho_eq * (pn - beq);
+                T wc = wr;
+                wc -= q.rho_eq * rw.yr;
+                ts.c.nEw = tmax(ts.c.nEw, tabs(Ed_next[i] * wc));
+                ts.c.lhs += beq * wc;
+                wyr[i] = Ed_next[i] * wr; wyc[i] = Ed_next[i] * wc;
+                test_close_column(ts, i, exn[i], wr, wc, fast_rcp(cy.Dx_next[i]));
+            }
+        }
+        if (TEST) {       // columns x_k and u_k get their rows dyn_{k+1}
+#pragma unroll
+            for (int j = 0; j < NX; ++j) {
+                T ar = 0, ac = 0;
+#pragma unroll
+                for (int i = 0; i < NX; ++i) { ar += m.A[i][j] * wyr[i]; ac += m.A[i][j] * wyc[i]; }
+                ownr_x[j] += Dx[j] * ar;
+                ownc_x[j] += Dx[j] * ac;
+            }
+#pragma unroll
+            for (int j = 0; j < NU; ++j) {
+                T ar = 0, ac = 0;
+#pragma unroll
+                for (int i = 0; i < NX; ++i) { ar += m.B[i][j] * wyr[i]; ac += m.B[i][j] * wyc[i]; }
+                T atyr = ownr_u[j], atyc = ownc_u[j];
+                atyr += Du[j] * ar;
+                atyc += Du[j] * ac;
+                const T Dinv = fast_rcp(Du[j]);
+                ts.r.dua = tmax(ts.r.dua, tabs(Dinv * (atyr + pxr_u[j])));
+                ts.r.nAty = tmax(ts.r.nAty, tabs(Dinv * atyr));
+                ts.c.nAty = tmax(ts.c.nAty, tabs(Dinv * atyc));
+            }
         }
 #pragma unroll
         for (int j = 0; j < NX; ++j) {
@@ -837,11 +1021,19 @@ MPCB_HD void admm_bwd_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const
     for (int a = 0; a < NW; ++a) MPCB_AT(R, L::R_T + a) = rh[a];
 #pragma unroll
     for (int i = 0; i < NX; ++i) { cy.xt_next[i] = w[i]; cy.Dx_next[i] = Dx[i]; }
+    if (TEST) {
+#pragma unroll
+        for (int i = 0; i < NX; ++i) {
+            ts.x_next[i] = xn_a[i]; ts.dx_next[i] = dx_a[i];
+            ts.own_r[i] = ownr_x[i]; ts.qpx_r[i] = qpx_x[i]; ts.own_c[i] = ownc_x[i];
+        }
+    }
 }
 
 // rows dyn_0 (header): updated after the backward sweep reached stage 0 (cy holds x~_0 and D_x(0))
-template <typename T, typename L, bool FIRST, bool SAVE>
-MPCB_HD void admm_bwd_header(const KParams<T>& p, const AdmmConst<T, L>& q, int b, T* H, const BwdCarry<T, L>& cy, T* O0) {
+template <typename T, typename L, bool FIRST, int MODE>
+MPCB_HD void admm_bwd_header(const KParams<T>& p, const AdmmConst<T, L>& q, int b, T* H, const BwdCarry<T, L>& cy,
+                             BwdTest<T, L>& ts) {
     constexpr bool first = FIRST;
 #pragma unroll
     for (int i = 0; i < L::NX; ++i) {
@@ -851,20 +1043,30 @@ MPCB_HD void admm_bwd_header(const KParams<T>& p, const AdmmConst<T, L>& q, int 
                                     q.rinv_eq());
         const T pn = row_next(-(E0 * cy.Dx_next[i]) * cy.xt_next[i], rw, q.alpha);
         MPCB_AT(H, L::H_P0 + i) = pn;
-        if (SAVE) MPCB_AT(O0, i) = pn;
+        if (MODE == kBwdTest) {     // rows dyn_0; column x_0 gets its row dyn_0
+            const T ex = E0 * cy.Dx_next[i], Einv = fast_rcp(E0);
+            const T axr = -ex * ts.x_next[i], axc = -ex * ts.dx_next[i];
+            ts.r.pri = tmax(ts.r.pri, tabs(Einv * (axr - beq)));
+            ts.r.nz = tmax(ts.r.nz, tabs(Einv * beq));
+            ts.r.nAx = tmax(ts.r.nAx, tabs(Einv * axr));
+            ts.c.aup = tmax(ts.c.aup, Einv * axc);
+            ts.c.alo = tmin(ts.c.alo, Einv * axc);
+            T wr = q.rho_eq * (pn - beq);
+            T wc = wr;
+            wc -= q.rho_eq * rw.yr;
+            ts.c.nEw = tmax(ts.c.nEw, tabs(E0 * wc));
+            ts.c.lhs += beq * wc;
+            test_close_column(ts, i, ex, wr, wc, fast_rcp(cy.Dx_next[i]));
+        }
     }
 }
 
-// ---- termination test on the unscaled residuals (auxil.c: check_termination), one stage
-template <typename T>
-struct Resid {
-    T pri, dua, nz, nAx, nq, nAty, nPx;
-};
 // Accumulators of the infeasibility certificates (auxil.c: is_primal_infeasible / is_dual_infeasible, paper
 // eq. (22), (24)) over delta_y = y^k - y^{k-1} and delta_x = x^k - x^{k-1} of the iteration being tested.  The
-// pre-update state of that iteration is copied by admm_save_old, before its forward sweep, into the old-state
-// buffer O (the Ruiz scratch, free after setup): [x (VS) | p (CS)] per stage, rows in the form they had then
-// (p-form; explicit z with y in the y rows on the first iteration of a solve).
+// backward sweep of a tested iteration (kBwdTest) forms them from the old state in the records it reads; the CTA and
+// dense kernels copy the pre-update state of that iteration into the old-state buffer O (the Ruiz scratch, free after
+// setup): [x (VS) | p (CS)] per stage, rows in the form they had then (p-form; explicit z with y in the y rows on the
+// first iteration of a solve).
 template <typename T>
 struct Cert {
     T ndy, lhs, nAtdy;            // ||E dy||_inf, u'max(dy,0) + l'min(dy,0), ||Dinv A'dy||_inf
@@ -887,39 +1089,17 @@ MPCB_HD T old_yr(bool first, T p_old, T y_old, T lb, T ub, T rho_row) {
     return p_old - tmin(tmax(p_old, lb), ub);
 }
 
-// ---- the termination sweep, one stage.  ONE body serves both evaluations OSQP makes at a termination test:
-//   cert = false: the residuals of (x, y)                          (auxil.c: compute_pri_res / compute_dua_res, tolerances)
-//   cert = true : the infeasibility certificates of (dx, dy) = (x - x_old, y - y_old)   (is_primal/dual_infeasible)
-// Both need the same linear forms — E^-1 A v by rows, D^-1 A'w and D^-1 P v by columns — applied to v = x, w = y or to
-// v = dx, w = dy, so the sweep is written over (v, w) and accumulates every norm either evaluation wants; the second
-// evaluation re-runs the same instructions instead of adding as many again (the kernel's code footprint, not its flop
-// count, is what the instruction cache of an SM with six warps at different places of a long unrolled loop feels).
-template <typename T>
-struct TestAcc {
-    T pri, dua, nz, nAx, nq, nAty, nPx;      // residual norms; nAty = ||D^-1 A'w||, nPx = ||D^-1 P v|| serve both evaluations
-    T nEw, lhs, nDv, qv, aup, alo;           // certificate terms: ||E w||, u'w+ + l'w-, ||D v||, q'v, max / min of E^-1 A v
-};
-template <typename T>
-MPCB_HD void test_reset(TestAcc<T>& a) {
-    a.pri = a.dua = a.nz = a.nAx = a.nq = a.nAty = a.nPx = 0;
-    a.nEw = a.lhs = a.nDv = a.qv = 0;
-    a.aup = (T)-kOsqpInfty; a.alo = (T)kOsqpInfty;
-}
+// ---- the termination sweep of the CTA and dense kernels, one stage: the terms of BwdTest as a sweep of its own over the new
+// state, once for each evaluation:
+//   cert = false: the residuals of (x, y)
+//   cert = true : the infeasibility certificates of (dx, dy), the old state read from the old-state buffer O
+// The second evaluation re-runs the same instructions instead of adding as many again (the kernel's code footprint, not
+// its flop count, is what the instruction cache of an SM with six warps at different places of a long unrolled loop
+// feels).  The column sums are associated like the backward sweep's (test_close_column).
 template <typename T, typename L>
 struct TestCarry {
     T Ed_cur[L::NX], wd_cur[L::NX];          // E and w of rows dyn_k
 };
-// is_primal_infeasible projects dy on the recession cone of the row's bound type first
-template <typename T>
-MPCB_HD T cert_project(bool inf_possible, T dy, T lb, T ub) {
-    if (inf_possible) {
-        const bool up_inf = ub > (T)(kOsqpInfty * kMinScaling), lo_inf = lb < (T)(-kOsqpInfty * kMinScaling);
-        if (up_inf && lo_inf) dy = 0;
-        else if (up_inf) dy = tmin(dy, (T)0);
-        else if (lo_inf) dy = tmax(dy, (T)0);
-    }
-    return dy;
-}
 
 template <typename T, typename L>
 MPCB_HD void admm_test_stage(const KParams<T>& p, const AdmmConst<T, L>& q, const Model<T, L>& m, int b, int k,
@@ -1031,9 +1211,11 @@ MPCB_HD void admm_test_stage(const KParams<T>& p, const AdmmConst<T, L>& q, cons
         T acc = 0;
 #pragma unroll
         for (int i = 0; i < NX; ++i) acc += m.A[i][j] * wy[i];
-        const T aty = -(cy.Ed_cur[j] * Dx[j]) * cy.wd_cur[j] + bx * wbx + (last ? (T)0 : Dx[j] * acc);
+        T aty = bx * wbx;
+        if (!last) aty += Dx[j] * acc;
+        aty -= (cy.Ed_cur[j] * Dx[j]) * cy.wd_cur[j];
         const T px = q.c * Qk[j] * Dx[j] * Dx[j] * vx[j];
-        t.dua = tmax(t.dua, tabs(Dinv * (qh + aty + px)));
+        t.dua = tmax(t.dua, tabs(Dinv * ((qh + px) + aty)));
         t.nq = tmax(t.nq, tabs(Dinv * qh));
         t.nAty = tmax(t.nAty, tabs(Dinv * aty));
         t.nPx = tmax(t.nPx, tabs(Dinv * px));
@@ -1074,7 +1256,8 @@ MPCB_HD void admm_test_stage(const KParams<T>& p, const AdmmConst<T, L>& q, cons
             T acc = 0;
 #pragma unroll
             for (int i = 0; i < NX; ++i) acc += m.B[i][j] * wy[i];
-            const T aty = bu * wbu + Du[j] * acc;
+            T aty = bu * wbu;
+            aty += Du[j] * acc;
             const T px = q.c * p.R[j] * Du[j] * Du[j] * vu[j];
             t.dua = tmax(t.dua, tabs(Dinv * (aty + px)));
             t.nAty = tmax(t.nAty, tabs(Dinv * aty));
