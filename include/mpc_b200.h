@@ -174,6 +174,12 @@ int mpcb_plant_step(int dtype, int batch, size_t ld, int nx, int nu, int shared_
  * last mpcb_setup/mpcb_update.  Element-major outputs (any may be NULL):
  *   Pdiag [nvar][ld], q [nvar][ld], Avals [nnz][ld] (CSC values, pattern below), l/u [ncon][ld] */
 int mpcb_build_qp(mpcb_solver* s, void* Pdiag, void* q, void* Avals, void* l, void* u, void* stream);
+/* The Ruiz scaling of the last mpcb_setup — OSQP's D, E and cost scaling c (scaling.c: scale_data) — for inspection and
+ * parity tests.  mpcb_update, mpcb_update_bounds and the solves keep it, like OSQP's update.  Batch-major DEVICE arrays
+ * in the reference's ordering, any pointer may be NULL:
+ *   D_out [batch][nvar] (x_0..x_N, u_0..u_{N-1}, s_0..s_N), E_out [batch][ncon] (dyn_0..dyn_N, bx_0..bx_N,
+ *   bu_0..bu_{N-1}), c_out [batch].  Returns MPCB_E_STATE before setup (or after settings that invalidate it). */
+int mpcb_get_scaling(mpcb_solver* s, void* D_out, void* E_out, void* c_out, void* stream);
 /* CSC pattern of A shared by the whole batch: Ap [nvar+1], Ai [nnz] (host arrays); returns nnz.
  * Pass NULLs to query nnz. */
 int mpcb_qp_pattern(const mpcb_solver* s, int* Ap, int* Ai);

@@ -85,6 +85,7 @@ _SIGNATURES = {
     "mpcb_plant_step": (C.c_int, [C.c_int, C.c_int, C.c_size_t, C.c_int, C.c_int, C.c_int, _VOIDP, _VOIDP, _VOIDP, _VOIDP, _VOIDP,
                                   C.c_int, _VOIDP, _VOIDP]),
     "mpcb_build_qp": (C.c_int, [_VOIDP, _VOIDP, _VOIDP, _VOIDP, _VOIDP, _VOIDP, _VOIDP]),
+    "mpcb_get_scaling": (C.c_int, [_VOIDP, _VOIDP, _VOIDP, _VOIDP, _VOIDP]),
     "mpcb_qp_pattern": (C.c_int, [_VOIDP, C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "mpcb_to_element_major": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_size_t, _VOIDP, _VOIDP, _VOIDP]),
     "mpcb_to_batch_major": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_size_t, _VOIDP, _VOIDP, _VOIDP]),

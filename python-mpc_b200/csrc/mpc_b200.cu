@@ -582,6 +582,13 @@ int mpcb_build_qp(mpcb_solver* s, void* Pdiag, void* q, void* Avals, void* l, vo
     return ops_of(s)->build_qp(s, &o, st);
 }
 
+int mpcb_get_scaling(mpcb_solver* s, void* D_out, void* E_out, void* c_out, void* stream) {
+    if (!s) return fail(MPCB_E_ARG, "null solver");
+    if (!s->is_setup) return fail(MPCB_E_STATE, "get_scaling before setup (or settings changed since setup)");
+    ScalingOut o{D_out, E_out, c_out};
+    return ops_of(s)->get_scaling(s, &o, (rt_stream)stream);
+}
+
 // ---- host front door ----------------------------------------------------------------------------
 static int ensure(void** p, size_t* have, size_t need) {
     if (*have >= need) return 0;

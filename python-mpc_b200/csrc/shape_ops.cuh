@@ -16,6 +16,11 @@ struct BuildOut {
     void *Pdiag, *q, *Avals, *l, *u;
 };
 
+// The Ruiz scalings in the reference's ordering (see mpcb_get_scaling in the header).
+struct ScalingOut {
+    void *D, *E, *c;
+};
+
 // entry points of one compiled (shape, dtype)
 struct ShapeOps {
     int nx, nu, slack, dtype;
@@ -24,6 +29,7 @@ struct ShapeOps {
     int (*run_admm)(mpcb_solver* s, int max_iter, int check_every, int warm, rt_stream st);
     int (*cold_start)(mpcb_solver* s, rt_stream st);
     int (*build_qp)(mpcb_solver* s, const BuildOut* o, rt_stream st);
+    int (*get_scaling)(mpcb_solver* s, const ScalingOut* o, rt_stream st);
 };
 
 // =============================================================================================
@@ -107,6 +113,44 @@ struct BuildFn {
     KParams<T> p;
     BuildOut o;
     MPCB_HD void operator()(int b) const { build_one<T, L>(p, o, b); }
+};
+
+// D, E, c of one QP from its home records and header, batch-major in the reference's ordering.  The slots without a
+// variable or row in the reference (u_N, dyn_{N+1} and bu_N of stage N) are skipped.
+template <typename T, typename L>
+MPCB_HD void scaling_one(const KParams<T>& p, const ScalingOut& o, int b) {
+    constexpr int NX = L::NX, NU = L::NU, NS = L::NS;
+    const int N = p.N;
+    const size_t nvar = (size_t)L::nvar(N), ncon = (size_t)L::ncon(N);
+    const size_t ux0 = (size_t)(N + 1) * NX, sx0 = ux0 + (size_t)N * NU;      // variable offsets
+    const size_t bx0 = (size_t)(N + 1) * NX, bu0 = 2 * (size_t)(N + 1) * NX;  // row offsets
+    T* D = o.D ? (T*)o.D + (size_t)b * nvar : nullptr;
+    T* E = o.E ? (T*)o.E + (size_t)b * ncon : nullptr;
+    const Ws<T, L> ws(p, b);
+    for (int k = 0; k <= N; ++k) {
+        const T* R = ws.R(k);
+        for (int j = 0; j < NX; ++j) {
+            if (D) D[(size_t)k * NX + j] = MPCB_AT(R, L::R_D + L::OX + j);
+            if (D && NS) D[sx0 + (size_t)k * NX + j] = MPCB_AT(R, L::R_D + L::OS + (NS ? j : 0));
+            if (E && k < N) E[(size_t)(k + 1) * NX + j] = MPCB_AT(R, L::R_E + L::ODN + j);
+            if (E) E[bx0 + (size_t)k * NX + j] = MPCB_AT(R, L::R_E + L::OBX + j);
+        }
+        if (k < N)
+            for (int j = 0; j < NU; ++j) {
+                if (D) D[ux0 + (size_t)k * NU + j] = MPCB_AT(R, L::R_D + L::OU + j);
+                if (E) E[bu0 + (size_t)k * NU + j] = MPCB_AT(R, L::R_E + L::OBU + j);
+            }
+    }
+    if (E)
+        for (int i = 0; i < NX; ++i) E[i] = MPCB_AT(ws.hdr, L::H_E0 + i);        // rows dyn_0 live in the header
+    if (o.c) ((T*)o.c)[b] = MPCB_AT(ws.hdr, L::H_C);
+}
+
+template <typename T, typename L>
+struct ScalingFn {
+    KParams<T> p;
+    ScalingOut o;
+    MPCB_HD void operator()(int b) const { scaling_one<T, L>(p, o, b); }
 };
 
 // osqp_update_bounds (osqp.c) + update_rho_vec (auxil.c) for one QP: did a bound row change its type between the old and
@@ -750,11 +794,16 @@ static int build_impl(mpcb_solver* s, const BuildOut* o, rt_stream st) {
     return launch_1d(p.B, st, BuildFn<T, L>{p, *o});
 }
 template <typename T, typename L>
+static int scaling_impl(mpcb_solver* s, const ScalingOut* o, rt_stream st) {
+    KParams<T> p = make_params<T>(s);
+    return launch_1d(p.B, st, ScalingFn<T, L>{p, *o});
+}
+template <typename T, typename L>
 static ShapeOps make_shape_ops() {
     ShapeOps o;
     o.nx = L::NX; o.nu = L::NU; o.slack = L::SLACK ? 1 : 0;
     o.dtype = std::is_same<T, float>::value ? MPCB_F32 : MPCB_F64;
     o.setup = &setup_impl<T, L>; o.refactor = &refactor_impl<T, L>; o.run_admm = &run_admm_impl<T, L>;
-    o.cold_start = &cold_impl<T, L>; o.build_qp = &build_impl<T, L>;
+    o.cold_start = &cold_impl<T, L>; o.build_qp = &build_impl<T, L>; o.get_scaling = &scaling_impl<T, L>;
     return o;
 }

@@ -309,6 +309,14 @@ class BatchSolver:
         out = [t[:, :B].t().contiguous() for t in (Pd, q, Av, l, u)]
         return out[0], out[1], out[2], out[3], out[4], Ap, Ai
 
+    def scaling(self):
+        """The Ruiz scaling of the last setup, OSQP's (D, E, c): D (B,nvar), E (B,ncon) in the reference's ordering, c (B,)."""
+        B = self.batch
+        mk = lambda *shape: torch.empty(shape, device=self.be.device, dtype=self.dtype)
+        D, E, c = mk(B, self.nvar), mk(B, self.ncon), mk(B)
+        self.be.check(self.be.lib.mpcb_get_scaling(self._h, ptr(D), ptr(E), ptr(c), self.be.stream()))
+        return D, E, c
+
     def solve_host(self, Ad, Bd, gd, x_init, Xr, want_x=True, want_u=True):
         """The host front door: numpy-layout HOST arrays in and out, copies inside (mpcb_solve_host)."""
         npdt = np.float32 if self.dtype == torch.float32 else np.float64
