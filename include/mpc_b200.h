@@ -171,7 +171,8 @@ int mpcb_plant_step(int dtype, int batch, size_t ld, int nx, int nu, int shared_
  * prob.setup()/prob.update() (mpc_kinematics.py:158-203, mpc_dynamics.py:163-245/300-396,
  * vehicle_lateral_mpc_slack_increment.py:79-115).  The solve path never materialises them; this
  * is for inspection, parity tests and users who want the QP itself.  Uses the stage data of the
- * last mpcb_setup/mpcb_update.  Element-major outputs (any may be NULL):
+ * last mpcb_setup/mpcb_update.  Infinite bounds come out as +-OSQP_INFTY (1e30), the values OSQP's
+ * Python interface passes on for them.  Element-major outputs (any may be NULL):
  *   Pdiag [nvar][ld], q [nvar][ld], Avals [nnz][ld] (CSC values, pattern below), l/u [ncon][ld] */
 int mpcb_build_qp(mpcb_solver* s, void* Pdiag, void* q, void* Avals, void* l, void* u, void* stream);
 /* The Ruiz scaling of the last mpcb_setup — OSQP's D, E and cost scaling c (scaling.c: scale_data) — for inspection and

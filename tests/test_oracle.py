@@ -161,6 +161,28 @@ def test_dynamics_model_restatement_equals_reference(golden):
         np.testing.assert_allclose(gd, g["dyn_gd"][i], rtol=0, atol=1e-11)
 
 
+def test_plant_step_and_kinematics_restatements_equal_reference(golden):
+    """oracle/vehicle_ref.py's dynamics_step, kinematics_model and kinematics_step vs the outputs of the reference's own
+    update_dynamics_model (low-speed guards included), get_kinematics_model and update_kinematics_model."""
+    from oracle import vehicle_ref
+    g = golden["vehicle_models"]
+    for i in range(g["dyn_x"].shape[0]):
+        xn, af, ar = vehicle_ref.dynamics_step(g["dyn_x"][i], g["dyn_u"][i], dt=float(g["dyn_dt"]))
+        np.testing.assert_allclose(xn, g["dyn_xnext"][i], rtol=0, atol=1e-12)
+        assert np.isfinite(af) and np.isfinite(ar)
+    for i in range(g["kin_x"].shape[0]):
+        A, B, C = vehicle_ref.kinematics_model(g["kin_x"][i], g["kin_u"][i], dt=float(g["kin_dt"]))
+        np.testing.assert_allclose(A, g["kin_A"][i], rtol=0, atol=1e-15)
+        np.testing.assert_allclose(B, g["kin_B"][i], rtol=0, atol=1e-15)
+        np.testing.assert_allclose(C, g["kin_C"][i], rtol=0, atol=1e-15)
+        xn = vehicle_ref.kinematics_step(g["kin_x"][i], g["kin_u"][i], dt=float(g["kin_dt"]))
+        np.testing.assert_allclose(xn, g["kin_xnext"][i], rtol=0, atol=1e-14)
+    # the yaw update sees the new speed: with the old one the fixture is missed wherever steer and acceleration are nonzero
+    x, u = g["kin_x"], g["kin_u"]
+    old = x[:, 3] + x[:, 2] / (1.25 + 1.40) * np.tan(u[:, 0]) * float(g["kin_dt"])
+    assert np.abs(old - g["kin_xnext"][:, 3]).max() > 1e-6
+
+
 def test_c_closed_loop_driver_reproduces_reference_script_fixture(golden):
     """oracle_closed_loop_batch (the CPU arm of bench.py's configs[4] record): setup once, update(l, u) + warm-started
     solve + plant step per scenario — against the closed-loop fixture of the reference script (H = 20 head) and, with a
